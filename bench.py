@@ -2,6 +2,7 @@
 
     python bench.py --gpus N --steps K --warmup W                      # this repo (sm_100a kernels)
     python bench.py --impl reference --gpus N --steps K --warmup W      # the reference's CPU path (oracle port)
+    python bench.py --gpus N --steps K --warmup W --dump-outputs DIR   # + the last timed step's outputs, DIR/<name>.npy
 
 A "step" is one full protected training step (experiments/image_generation.py:86-101): update_d + update_g
 with the black-box trigger / SSIM watermark loss and the white-box sign loss, global batch 512 split evenly over
@@ -44,7 +45,16 @@ def parse():
                          "cyclegan: BASELINE configs 3 / 4, one protected step of IPR-SRGAN (batch 16, 24 -> 96) / "
                          "IPR-CycleGAN (batch 1, 128 x 128) on the native networks (single GPU)")
     ap.add_argument("--samples", type=int, default=10000, help="--workload verify: trigger samples in the sweep")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (its metrics, the generated batch, "
+                         "the generator / discriminator state) as DIR/<name>.npy, float32 / float64, at most 64 MB: "
+                         "two builds run with the same arguments can then be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.workload != "step"):
+        ap.error("--dump-outputs is implemented for the protected training step (--impl b200 --workload step)")
+    return args
 
 
 def peaks():
@@ -169,11 +179,37 @@ def step_traffic():
         return None
 
 
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_step_outputs(out_dir, tr, metrics):
+    """What the last timed step left a caller, as out_dir/<name>.npy: every metric (float64), the generator and
+    discriminator state a checkpoint holds (float32; integer counters as float64) and the generated batch G(z)
+    (float32).  When the batch would take the total over DUMP_BYTES, a fixed seeded sample of its rows is written."""
+    import numpy as np
+    import torch
+    torch.cuda.synchronize()
+    arrays = {"metric." + k.replace("/", "."): np.float64(v) for k, v in metrics.items()}
+    for net in ("G", "D"):
+        for k, v in getattr(tr.model, net).state_dict().items():
+            v = v.detach().cpu()
+            arrays[net + "." + k] = v.numpy().astype(np.float32 if v.is_floating_point() else np.float64)
+    fake = tr.model.fake_sample.detach().float().cpu().numpy()
+    room = DUMP_BYTES - sum(a.nbytes + 1024 for a in arrays.values()) - 1024     # 1 KiB per .npy header, generously
+    if fake.nbytes > room:
+        keep = np.random.default_rng(0).choice(len(fake), room // fake[0].nbytes, replace=False)
+        fake = fake[np.sort(keep)]
+    arrays["fake_sample"] = fake
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    steps, warmup = max(1, min(args.steps, 40)), max(1, min(args.warmup, 3))
+    steps, warmup = args.steps, max(1, min(args.warmup, 3))
     sample = args.batch
     sps, dt, cores = cpu_reference_steps_per_sec(steps, warmup, sample)
     value = sps * sample / args.batch
@@ -285,6 +321,8 @@ def run_b200(args):
     e2e_ms = timed(e2e_step, args.steps)
     wall_e2e = time.perf_counter() - t0
     _dbg('e2e done')
+    if args.dump_outputs and rank == 0:
+        dump_step_outputs(args.dump_outputs, tr, metrics_box["m"])   # before the profiling step below moves the weights
     clocks = sampler.stop() if rank == 0 else None
 
     # live tensor-roofline measurement: one eager step with CUDA events around every GEMM launch
