@@ -71,6 +71,14 @@ int ipr_crop_postproc_f32(const float *x, float *out, const float *bg,
                           int64_t batch, int channels, int height, int width,
                           int size, int row0, int col0, ipr_stream_t stream);
 
+/* The same crop followed by out = clamp(crop, 0, 1): the post-processing of normalized=False outputs, which are already
+ * in data range 1 (the SRGAN family), before the per-sample SSIM and pHash of the verification loop
+ * (experiments/image_super_resolution.py:229).  Replaces apply_mask + clamp_(0, 1); NaN propagates and -0 stays -0
+ * as in torch.clamp.  Same arguments and error codes as ipr_crop_postproc_f32. */
+int ipr_crop_clamp01_f32(const float *x, float *out, const float *bg,
+                         int64_t batch, int channels, int height, int width,
+                         int size, int row0, int col0, ipr_stream_t stream);
+
 /* out = z; out[:, mask[j]] = constant.  Replaces RandomBitMask.forward (tools/random_bitmask.py:12-15).
  * mask: n int64 indices in [0, z_dim). */
 int ipr_bitmask_scatter_f32(const float *z, float *out, const int64_t *mask,

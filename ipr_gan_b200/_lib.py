@@ -41,6 +41,7 @@ SIGNATURES = {
                                      c_ptr, c_ptr, c_i64, c_ptr]),
     "ipr_crop_patch_f32": (c_int, [c_ptr, c_ptr, c_ptr, c_i64, c_int, c_int, c_int, c_int, c_int, c_int, c_ptr]),
     "ipr_crop_postproc_f32": (c_int, [c_ptr, c_ptr, c_ptr, c_i64, c_int, c_int, c_int, c_int, c_int, c_int, c_ptr]),
+    "ipr_crop_clamp01_f32": (c_int, [c_ptr, c_ptr, c_ptr, c_i64, c_int, c_int, c_int, c_int, c_int, c_int, c_ptr]),
     "ipr_bitmask_scatter_f32": (c_int, [c_ptr, c_ptr, c_ptr, c_i64, c_int, c_int, c_f32, c_ptr]),
     "ipr_transform_dist_f32": (c_int, [c_ptr, c_ptr, c_i64, c_ptr]),
     "ipr_transform_var_f32": (c_int, [c_ptr, c_ptr, c_ptr, c_ptr, c_i64, c_int, c_ptr]),

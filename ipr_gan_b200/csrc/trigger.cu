@@ -86,10 +86,15 @@ paste_scalar_kernel(const float *__restrict__ x, float *__restrict__ y, const fl
         xwm[i] = tdist_one(z[i]);
 }
 
-// POST: the evaluation loop's post-processing fused in -- out = (clamp(crop, -1, 1) + 1) / 2
-// (experiments/image_generation.py:141-149 `postproc`, applied to apply_mask's result): same three fp32 operations,
-// same order, so the uint8 conversion downstream sees bit-identical values.
-template <bool POST>
+// POST: the evaluation loop's post-processing fused in.
+//   CROP_PLAIN    apply_mask's result as is
+//   CROP_SIGNED   out = (clamp(crop, -1, 1) + 1) / 2 for normalized=True outputs (experiments/image_generation.py:141-149
+//                 `postproc`): same three fp32 operations, same order, so the uint8 conversion downstream sees
+//                 bit-identical values
+//   CROP_UNIT     out = clamp(crop, 0, 1) for normalized=False outputs, already in data range 1 (SRGAN)
+enum CropPost { CROP_PLAIN = 0, CROP_SIGNED = 1, CROP_UNIT = 2 };
+
+template <int POST>
 __global__ void __launch_bounds__(256)
 crop_kernel(const float *__restrict__ x, float *__restrict__ out, const float *__restrict__ bg,
             long long n_out, PasteGeom g)
@@ -104,10 +109,14 @@ crop_kernel(const float *__restrict__ x, float *__restrict__ out, const float *_
         const float v = x[((size_t)plane * g.H + (hh + g.row0)) * g.W + (cc + g.col0)];
         // y = ones * bg ; y += (1 - bg) * crop      (tools/paste_watermark.py:58-60)
         float r = __fadd_rn(__fmul_rn(1.0f, b), __fmul_rn(__fsub_rn(1.0f, b), v));
-        if (POST) {
-            // torch.clamp propagates NaN; fminf / fmaxf would drop it
+        // torch.clamp propagates NaN; fminf / fmaxf would drop it
+        if (POST == CROP_SIGNED) {
             r = (r != r) ? r : fminf(fmaxf(r, -1.0f), 1.0f);
             r = __fmul_rn(__fadd_rn(r, 1.0f), 0.5f);
+        } else if (POST == CROP_UNIT) {
+            // torch.clamp's min(max(v, lo), hi) with the comparisons spelled out: NaN passes, -0 stays -0
+            r = (r < 0.0f) ? 0.0f : r;
+            r = (r > 1.0f) ? 1.0f : r;
         }
         out[i] = r;
     }
@@ -203,32 +212,43 @@ extern "C" int ipr_trigger_pair_f32(const float *x, float *ywm, const float *fg,
                       ipr_cu(stream));
 }
 
-extern "C" int ipr_crop_patch_f32(const float *x, float *out, const float *bg,
-                                  int64_t batch, int channels, int height, int width,
-                                  int size, int row0, int col0, ipr_stream_t stream)
+namespace {
+
+template <int POST>
+int crop_impl(const float *x, float *out, const float *bg, int64_t batch, int channels, int height, int width,
+              int size, int row0, int col0, cudaStream_t st)
 {
     IPR_REQUIRE(x && out && bg, IPR_E_NULL);
     IPR_REQUIRE(batch > 0 && channels > 0 && height > 0 && width > 0 && size > 0, IPR_E_SHAPE);
     IPR_REQUIRE(row0 >= 0 && col0 >= 0 && row0 + size <= height && col0 + size <= width, IPR_E_SHAPE);
     PasteGeom g{channels, height, width, size, row0, col0};
     const long long n = (long long)batch * channels * size * size;
-    crop_kernel<false><<<grid_for(n, 256), 256, 0, ipr_cu(stream)>>>(x, out, bg, n, g);
+    crop_kernel<POST><<<grid_for(n, 256), 256, 0, st>>>(x, out, bg, n, g);
     IPR_LAUNCH_CHECK();
     return IPR_OK;
+}
+
+}  // namespace
+
+extern "C" int ipr_crop_patch_f32(const float *x, float *out, const float *bg,
+                                  int64_t batch, int channels, int height, int width,
+                                  int size, int row0, int col0, ipr_stream_t stream)
+{
+    return crop_impl<CROP_PLAIN>(x, out, bg, batch, channels, height, width, size, row0, col0, ipr_cu(stream));
 }
 
 extern "C" int ipr_crop_postproc_f32(const float *x, float *out, const float *bg,
                                      int64_t batch, int channels, int height, int width,
                                      int size, int row0, int col0, ipr_stream_t stream)
 {
-    IPR_REQUIRE(x && out && bg, IPR_E_NULL);
-    IPR_REQUIRE(batch > 0 && channels > 0 && height > 0 && width > 0 && size > 0, IPR_E_SHAPE);
-    IPR_REQUIRE(row0 >= 0 && col0 >= 0 && row0 + size <= height && col0 + size <= width, IPR_E_SHAPE);
-    PasteGeom g{channels, height, width, size, row0, col0};
-    const long long n = (long long)batch * channels * size * size;
-    crop_kernel<true><<<grid_for(n, 256), 256, 0, ipr_cu(stream)>>>(x, out, bg, n, g);
-    IPR_LAUNCH_CHECK();
-    return IPR_OK;
+    return crop_impl<CROP_SIGNED>(x, out, bg, batch, channels, height, width, size, row0, col0, ipr_cu(stream));
+}
+
+extern "C" int ipr_crop_clamp01_f32(const float *x, float *out, const float *bg,
+                                    int64_t batch, int channels, int height, int width,
+                                    int size, int row0, int col0, ipr_stream_t stream)
+{
+    return crop_impl<CROP_UNIT>(x, out, bg, batch, channels, height, width, size, row0, col0, ipr_cu(stream));
 }
 
 extern "C" int ipr_bitmask_scatter_f32(const float *z, float *out, const int64_t *mask,

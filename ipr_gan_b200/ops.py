@@ -66,16 +66,28 @@ def trigger_pair(x, fg, bg, position, size, z):
     return xwm, y
 
 
+_CROP_FNS = {False: "ipr_crop_patch_f32", True: "ipr_crop_postproc_f32", "signed": "ipr_crop_postproc_f32",
+             "unit": "ipr_crop_clamp01_f32"}
+
+
+def postproc_mode(normalized):
+    """The evaluation loop's post-processing for a trigger's ``normalized`` flag: 'signed' maps [-1, 1] outputs to
+    [0, 1] with (clamp(-1, 1) + 1) / 2, 'unit' clamps outputs that are already in data range 1 to [0, 1]."""
+    return "signed" if normalized else "unit"
+
+
 def crop_patch(x, bg, position, size, postproc=False):
-    """apply_mask's crop; ``postproc``: followed by (clamp(-1, 1) + 1) / 2 in the same launch (the evaluation loop)."""
+    """apply_mask's crop, optionally followed in the same launch by the evaluation loop's post-processing:
+    ``postproc`` False: none; True or 'signed': (clamp(-1, 1) + 1) / 2; 'unit': clamp(0, 1) (see postproc_mode)."""
+    if postproc not in _CROP_FNS:
+        raise IprError("crop_patch: postproc must be False, True, 'signed' or 'unit', got %r" % (postproc,))
     x = _req(x, "x")
     bg = _req(bg, "bg")
     B, C, H, W = x.shape
     r0, c0 = window_origin(position, size, H, W)
     out = torch.empty(B, C, size, size, device=x.device, dtype=x.dtype)
-    fn = lib().ipr_crop_postproc_f32 if postproc else lib().ipr_crop_patch_f32
-    check(fn(_p(x), _p(out), _p(bg), B, C, H, W, size, r0, c0, _stream()),
-          "ipr_crop_postproc_f32" if postproc else "ipr_crop_patch_f32")
+    name = _CROP_FNS[postproc]
+    check(getattr(lib(), name)(_p(x), _p(out), _p(bg), B, C, H, W, size, r0, c0, _stream()), name)
     return out
 
 
