@@ -286,6 +286,15 @@ int ipr_im2col3_bf16(const float *x, const float *tanh_out, void *out, int64_t b
 int ipr_col2im3_f32(const float *t, float *out, int64_t batch, int height, int width, int ld, int tanh_out,
                     ipr_stream_t stream);
 
+/* The same layer in ONE launch, without the tap tensor: a = (batch, height, width, 64) bf16 NHWC (16-byte aligned),
+ * b = the [1][32][64] bf16 tap pack (row (kh*3+kw)*3 + c, column = input channel; 16-byte aligned), sigma optional
+ * (device scalar: the taps are divided by it), out = (batch, 3, height, width) fp32.  Bit-identical to
+ * ipr_tapgemm_bf16 (linear, IPR_EPI_LINEAR_F32, n_total 32) followed by ipr_col2im3_f32.  One CTA folds whole images
+ * in shared memory: height*width must be a multiple of 128 and at most 1024, and width must divide 128
+ * (else IPR_E_UNSUPPORTED, and the caller keeps the two-launch path). */
+int ipr_tapfold3_f32(const void *a, const void *b, const float *sigma, float *out, int64_t batch, int height,
+                     int width, int tanh_out, ipr_stream_t stream);
+
 /* BatchNorm2d training-mode statistics (networks/conv_generator.py:9): partial = [rows][2][C] column sums and
  * sums of squares produced by the GEMM epilogue; count = elements per channel.  Writes scale = gamma*rstd,
  * shift = beta - mean*scale, mean, rstd and (if running_mean != NULL) updates the running statistics with

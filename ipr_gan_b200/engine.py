@@ -58,6 +58,29 @@ def col2im3(t, tanh_out):
     return out
 
 
+IPR_E_UNSUPPORTED = -3
+
+
+def tapfold3(a, b_packed, tanh_out, sigma=None):
+    """The 3-output-channel 3x3 layer in one launch (csrc/tapfold.cu): a (B, H, W, 64) bf16 NHWC, b_packed the
+    [1][32][64] ``_tap27_rows_layout`` pack -> (B, 3, H, W) fp32, bit-identical to ``col2im3`` of the tap GEMM.
+    Returns None where the kernel does not cover the shape, or with IPR_NO_TAPFOLD=1 (A/B runs); the caller then
+    runs the tap GEMM + ``col2im3``."""
+    if os.environ.get("IPR_NO_TAPFOLD", "0") != "0":
+        return None
+    B, H, W, C = a.shape
+    assert C == 64 and a.dtype == torch.bfloat16 and a.is_contiguous() and b_packed.dtype == torch.bfloat16
+    out = torch.empty(B, 3, H, W, device=a.device, dtype=torch.float32)
+    ev = dense._prof_begin()
+    rc = lib().ipr_tapfold3_f32(_p(a), _p(b_packed), _p(sigma), _p(out), B, H, W, int(bool(tanh_out)), _st())
+    if rc == IPR_E_UNSUPPORTED:
+        return None
+    check(rc, "ipr_tapfold3_f32")
+    # the tap GEMM's useful flops (27 of 32 columns); the fold's adds are not counted
+    dense._prof_end("tapfold:3ch", 2.0 * B * H * W * 64 * 27, ev, B * H * W * 128.0 + b_packed.numel() * 2)
+    return out
+
+
 def colsum_partials(partial, out=None, accumulate=False, scale=1.0, ncols=None):
     """partial: [rows][row_stride] fp32 -> out[ncols] = column sums of the first ``ncols`` columns (fixed order)."""
     rows, stride = partial.shape[0], partial.numel() // partial.shape[0]
@@ -578,8 +601,10 @@ class _GeneratorFn(torch.autograd.Function):
             rstds.append(rstd)
             scales.append(scale)
             shifts.append(shift)
-        t9, _ = P.last.run(acts[-1], P.packs.get("ct3"), epi=dense.EPI_LINEAR_F32, n_valid=32)
-        out = col2im3(t9, True)
+        out = tapfold3(acts[-1], P.packs.get("ct3"), True)
+        if out is None:
+            t9, _ = P.last.run(acts[-1], P.packs.get("ct3"), epi=dense.EPI_LINEAR_F32, n_valid=32)
+            out = col2im3(t9, True)
         if CAPTURE_ACTS is not None:
             CAPTURE_ACTS.append(("G", list(acts)))
         ctx.module = module
@@ -753,8 +778,10 @@ class _DiscriminatorFn(torch.autograd.Function):
                          st, dst, key=2 + i)
         dx = None
         if ctx.x_needs_grad:
-            t9, _ = P.first_dg.run(dy, P.packs.get("c0_dg"), epi=dense.EPI_LINEAR_F32, sigma=sig[0], n_valid=32)
-            dx = col2im3(t9, False)
+            dx = tapfold3(dy, P.packs.get("c0_dg"), False, sigma=sig[0])
+            if dx is None:
+                t9, _ = P.first_dg.run(dy, P.packs.get("c0_dg"), epi=dense.EPI_LINEAR_F32, sigma=sig[0], n_valid=32)
+                dx = col2im3(t9, False)
         if want:
             gW[0] = torch.empty_like(ws[0])
             fork.run(lambda: P.first_wg.run(dy, col, gW[0]), dy, key=0)
