@@ -295,6 +295,16 @@ int ipr_col2im3_f32(const float *t, float *out, int64_t batch, int height, int w
 int ipr_tapfold3_f32(const void *a, const void *b, const float *sigma, float *out, int64_t batch, int height,
                      int width, int tanh_out, ipr_stream_t stream);
 
+/* The same layer, same arguments and same results, for larger images: ConvTranspose2d(64,3,3,1,1)+Tanh of
+ * networks/conv_generator.py:21-22 and the input gradient of Conv2d(3,64,3,1,1) of networks/sn_discriminator.py:15
+ * in the 64 x 64 networks (mg = md = 8), which the entry point above hands back.  A work item is a band of output
+ * rows of one image: it stages the taps of its rows and of the rows above and below (recomputed from whole,
+ * GEMM-aligned 128-row sub-tiles) and folds them.  Rows per band are chosen per shape (64 x 64: 12).  height*width must be a multiple of 128, width
+ * must divide 128 and be at most 128 (else IPR_E_UNSUPPORTED, and the caller keeps the two-launch path); images of
+ * 1024 pixels and fewer are accepted too. */
+int ipr_tapfold3_band_f32(const void *a, const void *b, const float *sigma, float *out, int64_t batch, int height,
+                          int width, int tanh_out, ipr_stream_t stream);
+
 /* BatchNorm2d training-mode statistics (networks/conv_generator.py:9): partial = [rows][2][C] column sums and
  * sums of squares produced by the GEMM epilogue; count = elements per channel.  Writes scale = gamma*rstd,
  * shift = beta - mean*scale, mean, rstd and (if running_mean != NULL) updates the running statistics with

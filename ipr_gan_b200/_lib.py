@@ -64,6 +64,7 @@ SIGNATURES = {
     "ipr_im2col3_bf16": (c_int, [c_ptr, c_ptr, c_ptr, c_i64, c_int, c_int, c_ptr]),
     "ipr_col2im3_f32": (c_int, [c_ptr, c_ptr, c_i64, c_int, c_int, c_int, c_int, c_ptr]),
     "ipr_tapfold3_f32": (c_int, [c_ptr, c_ptr, c_ptr, c_ptr, c_i64, c_int, c_int, c_int, c_ptr]),
+    "ipr_tapfold3_band_f32": (c_int, [c_ptr, c_ptr, c_ptr, c_ptr, c_i64, c_int, c_int, c_int, c_ptr]),
     "ipr_bn_finalize_f32": (c_int, [c_ptr, c_int, c_int, ctypes.c_double, c_f32, c_f32, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr]),
     "ipr_bn_apply_relu_bf16": (c_int, [c_ptr, c_ptr, c_ptr, c_ptr, c_i64, c_int, c_ptr]),
     "ipr_bn_bwd_workspace_bytes": (c_size, [c_int]),

@@ -81,6 +81,33 @@ def tapfold3(a, b_packed, tanh_out, sigma=None):
     return out
 
 
+def tapfold3_band(a, b_packed, tanh_out, sigma=None):
+    """``tapfold3`` for images larger than one CTA stages (the 64 x 64 networks): the kernel folds bands of output
+    rows, recomputing the GEMM-aligned sub-tile above and below each band for its halo rows, with the same results.
+    Returns None where the kernel does not cover the shape, or with IPR_NO_TAPFOLD=1; the caller then runs the tap
+    GEMM + ``col2im3``."""
+    if os.environ.get("IPR_NO_TAPFOLD", "0") != "0":
+        return None
+    B, H, W, C = a.shape
+    assert C == 64 and a.dtype == torch.bfloat16 and a.is_contiguous() and b_packed.dtype == torch.bfloat16
+    out = torch.empty(B, 3, H, W, device=a.device, dtype=torch.float32)
+    ev = dense._prof_begin()
+    rc = lib().ipr_tapfold3_band_f32(_p(a), _p(b_packed), _p(sigma), _p(out), B, H, W, int(bool(tanh_out)), _st())
+    if rc == IPR_E_UNSUPPORTED:
+        return None
+    check(rc, "ipr_tapfold3_band_f32")
+    # counted as tapfold3 counts: the sub-tiles a band re-reads for its halo rows (a third more A at 64 x 64) are not
+    dense._prof_end("tapfold:3ch", 2.0 * B * H * W * 64 * 27, ev, B * H * W * 128.0 + b_packed.numel() * 2)
+    return out
+
+
+def _fold3(a, b_packed, tanh_out, sigma=None):
+    """The 3-output-channel 3x3 layer as one launch where a kernel covers the shape: whole images, then bands.
+    None: the caller runs the tap GEMM + ``col2im3``."""
+    out = tapfold3(a, b_packed, tanh_out, sigma=sigma)
+    return out if out is not None else tapfold3_band(a, b_packed, tanh_out, sigma=sigma)
+
+
 def colsum_partials(partial, out=None, accumulate=False, scale=1.0, ncols=None):
     """partial: [rows][row_stride] fp32 -> out[ncols] = column sums of the first ``ncols`` columns (fixed order)."""
     rows, stride = partial.shape[0], partial.numel() // partial.shape[0]
@@ -601,7 +628,7 @@ class _GeneratorFn(torch.autograd.Function):
             rstds.append(rstd)
             scales.append(scale)
             shifts.append(shift)
-        out = tapfold3(acts[-1], P.packs.get("ct3"), True)
+        out = _fold3(acts[-1], P.packs.get("ct3"), True)
         if out is None:
             t9, _ = P.last.run(acts[-1], P.packs.get("ct3"), epi=dense.EPI_LINEAR_F32, n_valid=32)
             out = col2im3(t9, True)
@@ -778,7 +805,7 @@ class _DiscriminatorFn(torch.autograd.Function):
                          st, dst, key=2 + i)
         dx = None
         if ctx.x_needs_grad:
-            dx = tapfold3(dy, P.packs.get("c0_dg"), False, sigma=sig[0])
+            dx = _fold3(dy, P.packs.get("c0_dg"), False, sigma=sig[0])
             if dx is None:
                 t9, _ = P.first_dg.run(dy, P.packs.get("c0_dg"), epi=dense.EPI_LINEAR_F32, sigma=sig[0], n_valid=32)
                 dx = col2im3(t9, False)

@@ -34,7 +34,8 @@ from ipr_gan_b200 import _lib, engine  # noqa: E402
 
 class ProtectedDCGANTrainer(object):
     def __init__(self, batch, device, seed=1234, fn_inp="TransformDist", use_graph=True, size=32,
-                 device_latents=False, pinned_inputs=False):
+                 device_latents=False, pinned_inputs=False, wm_size=16):
+        # size / wm_size: 32 / 16 for the CIFAR configs, 64 / 32 for the CUB-200 ones (SURVEY.md section 8a, A4)
         self.batch, self.device, self.use_graph = batch, device, use_graph
         self.device_latents = device_latents
         # pinned_inputs: a second graph whose first nodes are the host->device copies of the step's batch out of the
@@ -48,7 +49,7 @@ class ProtectedDCGANTrainer(object):
         if use_graph:
             mcfg.opt_param["capturable"] = True
         model = models.DCGAN(mcfg, device=[device])
-        model = models.BlackBoxWrapper(model, presets.dcgan_blackbox(fn_inp=fn_inp))
+        model = models.BlackBoxWrapper(model, presets.dcgan_blackbox(fn_inp=fn_inp, wm_size=wm_size))
         model = models.WhiteBoxWrapper(model, presets.dcgan_whitebox())
         self.model = model
         self.real = torch.zeros(batch, 3, size, size, device=device)
