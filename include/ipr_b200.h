@@ -468,6 +468,27 @@ int ipr_norm_bwd_bf16(const void *dy, const void *x, void *dx, int groups, int64
                       float sign_scale, int act, float slope, const float *slope_ptr, float *dslope, void *workspace,
                       size_t workspace_bytes, ipr_stream_t stream);
 
+/* ------------------------------------------------------------------ robustness attacks (csrc/prune.cu)
+ * Global magnitude pruning, in place, over the N = n_total entries of a list of segments of an fp32 parameter
+ * arena: the removal attack of the reference's prune.py (SURVEY.md 2.1 row 34), i.e.
+ * torch.nn.utils.prune.global_unstructured(..., pruning_method=L1Unstructured, amount) with k = round(amount * N).
+ *   segments: device table of n_segments (offset, count) int64 pairs, offsets ascending, segments disjoint,
+ *             counts > 0 summing to n_total (8-byte aligned; n_segments <= IPR_PRUNE_MAX_SEGMENTS);
+ *   exactly k entries are zeroed, those with the smallest |w| over all segments together; a zeroed entry becomes
+ *   w * 0 (a negative weight becomes -0.0: bit-identical to weight_orig * weight_mask); +-0 share the key 0 and
+ *   every NaN ranks above every finite value and +inf (torch.topk's order);
+ *   ties at the k-th magnitude, whose order torch leaves unspecified: the lowest arena index is pruned first;
+ *   k = 0 launches nothing, k = N zeroes every segment entry; entries outside the segments are never written.
+ * The threshold is selected on the device (radix select), nothing is read back: the launches are graph-capturable.
+ * workspace: ipr_prune_workspace_bytes(n_total) bytes, 256-byte aligned. */
+#define IPR_PRUNE_MAX_SEGMENTS 256
+size_t ipr_prune_workspace_bytes(int64_t n_total);
+int ipr_prune_magnitude_f32(float *arena, const int64_t *segments, int n_segments, int64_t n_total, int64_t k,
+                            void *workspace, size_t workspace_bytes, ipr_stream_t stream);
+/* arena[index[i]] = -arena[index[i]] for i < n, indices distinct (device int64 list): the sign flip of
+ * normalisation gammas of the ambiguity attack (sign_flip.py:59-77).  One launch; n = 0 launches nothing. */
+int ipr_negate_indexed_f32(float *arena, const int64_t *index, int64_t n, ipr_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -100,6 +100,9 @@ SIGNATURES = {
     "ipr_wgrad_reduce_f32": (c_int, [c_ptr, c_int, c_int, c_int, c_int, c_ptr, c_ptr, c_i64, c_ptr, c_int, c_f32, c_ptr]),
     "ipr_wgrad_reduce_taps_f32": (c_int, [c_ptr, c_int, c_int, c_int, c_int, c_int, c_ptr, c_int, c_i64, c_i64, c_ptr, c_int,
                                           ctypes.c_float, c_ptr]),
+    "ipr_prune_workspace_bytes": (c_size, [c_i64]),
+    "ipr_prune_magnitude_f32": (c_int, [c_ptr, c_ptr, c_int, c_i64, c_i64, c_ptr, c_size, c_ptr]),
+    "ipr_negate_indexed_f32": (c_int, [c_ptr, c_ptr, c_i64, c_ptr]),
 }
 
 _lib = None

@@ -16,8 +16,8 @@ kernels of csrc/nn_misc.cu.  Nothing here synchronises or allocates outside PyTo
 allocator, so a whole training step can be captured in one CUDA graph.
 """
 import ctypes
-
 import os
+import weakref
 
 import torch
 
@@ -211,13 +211,7 @@ class PackSet(object):
     gather launch (csrc/optim.cu) whenever the masters changed."""
 
     def __init__(self, module, specs, specs_f32=()):
-        # the arena the parameters already live in (an optimizer may have built one spanning several networks, e.g.
-        # CycleGAN's optG over both generators), else one for this network alone
-        params = list(module.parameters())
-        arena = flat.arena_of(params[0])
-        if arena is None or any(flat.arena_of(p) is not arena for p in params):
-            arena = flat.arena_for(params)
-        self.arena = arena
+        self.arena = flat.module_arena(module)
         dev = self.arena.param.device
         # fp32 side table: permuted fp32 copies (Linear bias in NHWC feature order, the final GEMV row), same launch
         parts32, self.slices32, off32 = [], {}, 0
@@ -563,6 +557,27 @@ def _mark_dirty(module):
         a.clean = False
 
 
+_PARAM_DICTS = weakref.WeakKeyDictionary()     # network -> its modules' (parameter dict, buffer dict) pairs
+
+
+def refuse_pruned(net):
+    """Raise when a module of the network carries a ``torch.nn.utils.prune`` reparametrisation (a ``<name>_orig``
+    parameter next to a ``<name>_mask`` buffer).  The native forward never calls the children, so prune's pre-hook
+    that recomputes ``<name> = <name>_orig * <name>_mask`` never runs, and the packed operands are gathered from the
+    arena slot of the original parameter: a forward would silently use the unpruned weights (or, with plans built
+    after pruning, fail to find ``<name>`` in any arena)."""
+    dicts = _PARAM_DICTS.get(net)
+    if dicts is None:                   # the dicts themselves are never replaced: prune edits them in place
+        dicts = _PARAM_DICTS[net] = tuple((m._parameters, m._buffers) for m in net.modules() if m._parameters)
+    for params, buffers in dicts:
+        for name in params:
+            if name[-5:] == "_orig" and name[:-5] + "_mask" in buffers:
+                from .ops import IprError
+                raise IprError("%s: parameter %r is reparametrised by torch.nn.utils.prune, which the native forward "
+                               "cannot honour; prune the arena in place with ipr_gan_b200.robustness.prune_ instead "
+                               "(and torch.nn.utils.prune.remove() this one)" % (type(net).__name__, name))
+
+
 def _plans(module, cls):
     p = getattr(module, "_ipr_plans", None)
     if p is not None:
@@ -697,6 +712,7 @@ class _GeneratorFn(torch.autograd.Function):
 
 
 def generator_forward(module, z):
+    refuse_pruned(module)
     z = z.to(device=module.fc[0].weight.device, dtype=torch.float32)
     c = module.convs
     return _GeneratorFn.apply(module, z, module.fc[0].weight, module.fc[0].bias,
@@ -837,6 +853,7 @@ class _DiscriminatorFn(torch.autograd.Function):
 
 
 def discriminator_forward(module, x):
+    refuse_pruned(module)
     layers = _sn_layers(module)
     x = x.to(device=layers[0].weight_orig.device, dtype=torch.float32)
     params = []

@@ -94,6 +94,16 @@ def arena_for(params):
     return Arena(params)
 
 
+def module_arena(module):
+    """The arena a network's parameters live in (an optimizer may have built one spanning several networks, e.g.
+    CycleGAN's optG over both generators), else one for this network alone."""
+    params = list(module.parameters())
+    arena = arena_of(params[0])                 # validates the arena once; the lookups below are then O(1) each
+    if arena is None or any(_BY_PARAM.get(id(p)) is not arena for p in params):
+        arena = arena_for(params)
+    return arena
+
+
 def arena_of(param):
     hit = _BY_PARAM.get(id(param))
     return hit if hit is not None and hit.valid() else None

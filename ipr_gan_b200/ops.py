@@ -355,3 +355,31 @@ def unpack_hash_bits(h):
     """(B, 8) int32 words -> (B, 256) uint8 bits, bit k = 16*i + j of the DCT block (host helper for tests)."""
     words = h.detach().cpu().numpy().astype(np.uint32)
     return ((words[:, :, None] >> np.arange(32, dtype=np.uint32)[None, None, :]) & 1).reshape(words.shape[0], 256).astype(np.uint8)
+
+
+# ------------------------------------------------------------------------------ robustness attacks
+def prune_magnitude_(arena, segments, n_total, k):
+    """Global magnitude pruning in place (csrc/prune.cu): zero the k entries of smallest |w| over the ``segments`` of
+    the flat fp32 ``arena`` (ties: lowest index first).  segments: (S, 2) int64 CUDA tensor of ascending, disjoint
+    (offset, count) rows whose counts sum to ``n_total``.  Nothing is read back: graph-capturable."""
+    if not isinstance(arena, torch.Tensor) or not arena.is_cuda or arena.dtype != torch.float32 or not arena.is_contiguous():
+        raise IprError("arena must be a contiguous float32 CUDA tensor (it is pruned in place)")
+    segments = _req(segments, "segments", torch.int64)
+    if segments.dim() != 2 or segments.shape[1] != 2 or segments.device != arena.device:
+        raise IprError("segments must be an (S, 2) int64 tensor on the arena's device")
+    nbytes = lib().ipr_prune_workspace_bytes(int(n_total))
+    ws = torch.empty(max(1, nbytes), device=arena.device, dtype=torch.uint8)
+    check(lib().ipr_prune_magnitude_f32(_p(arena), _p(segments), segments.shape[0], int(n_total), int(k), _p(ws), nbytes,
+                                        _stream()), "ipr_prune_magnitude_f32")
+    return arena
+
+
+def negate_indexed_(arena, index):
+    """arena[index] = -arena[index] in one launch (distinct int64 CUDA indices)."""
+    if not isinstance(arena, torch.Tensor) or not arena.is_cuda or arena.dtype != torch.float32 or not arena.is_contiguous():
+        raise IprError("arena must be a contiguous float32 CUDA tensor (it is changed in place)")
+    index = _req(index, "index", torch.int64)
+    if index.device != arena.device:
+        raise IprError("index must be on the arena's device")
+    check(lib().ipr_negate_indexed_f32(_p(arena), _p(index), index.numel(), _stream()), "ipr_negate_indexed_f32")
+    return arena

@@ -445,5 +445,6 @@ class _SeqFn(torch.autograd.Function):
 
 def forward(net, x):
     """What the drop-in modules' ``forward`` calls on CUDA."""
+    engine.refuse_pruned(net)
     x = x.to(device=next(net.parameters()).device, dtype=torch.float32)
     return _SeqFn.apply(net, x, *list(net.parameters()))
