@@ -16,6 +16,7 @@ c_ptr = ctypes.c_void_p
 c_size = ctypes.c_size_t
 
 SIGN_MAX_LAYERS = 64
+MAX_TAPS, MAX_PHASES = 16, 4          # IPR_TG_MAX_TAPS, IPR_TG_MAX_PHASES
 
 
 class SnLayer(ctypes.Structure):
@@ -29,6 +30,38 @@ class SignLayer(ctypes.Structure):
     """ipr_sign_layer_t"""
     _fields_ = [("gamma", c_ptr), ("sign", c_ptr), ("grad", c_ptr), ("n", ctypes.c_int32),
                 ("reserved", ctypes.c_int32)]
+
+
+class TapGemm(ctypes.Structure):
+    """ipr_tapgemm_t"""
+    _fields_ = [
+        ("a", c_ptr), ("a_n", ctypes.c_int32), ("a_h", ctypes.c_int32), ("a_w", ctypes.c_int32),
+        ("a_c", ctypes.c_int32), ("a_parity", ctypes.c_int32), ("q_h", ctypes.c_int32), ("q_w", ctypes.c_int32),
+        ("b", c_ptr), ("n_total", ctypes.c_int32), ("block_n", ctypes.c_int32),
+        ("n_phases", ctypes.c_int32), ("n_taps", ctypes.c_int32),
+        ("tap_map", (ctypes.c_int8 * MAX_TAPS) * MAX_PHASES), ("tap_dh", (ctypes.c_int8 * MAX_TAPS) * MAX_PHASES),
+        ("tap_dw", (ctypes.c_int8 * MAX_TAPS) * MAX_PHASES),
+        ("epi_mode", ctypes.c_int32), ("slope", ctypes.c_float), ("sigma", c_ptr),
+        ("bias", c_ptr), ("mask", c_ptr), ("out", c_ptr),
+        ("out_h", ctypes.c_int32), ("out_w", ctypes.c_int32), ("out_c", ctypes.c_int32),
+        ("out_sh", ctypes.c_int32), ("out_sw", ctypes.c_int32),
+        ("out_oh", ctypes.c_int8 * MAX_PHASES), ("out_ow", ctypes.c_int8 * MAX_PHASES),
+        ("n_valid", ctypes.c_int32), ("stats", c_ptr), ("scale", c_ptr),
+    ]
+
+
+class WGrad(ctypes.Structure):
+    """ipr_wgrad_t"""
+    _fields_ = [
+        ("y", c_ptr), ("y_c", ctypes.c_int32), ("y_parity", ctypes.c_int32),
+        ("x", c_ptr), ("x_c", ctypes.c_int32), ("x_parity", ctypes.c_int32),
+        ("n_imgs", ctypes.c_int32), ("q_h", ctypes.c_int32), ("q_w", ctypes.c_int32),
+        ("n_phases", ctypes.c_int32), ("n_taps", ctypes.c_int32),
+        ("y_map", ctypes.c_int8 * MAX_PHASES),
+        ("tap_map", (ctypes.c_int8 * MAX_TAPS) * MAX_PHASES), ("tap_dh", (ctypes.c_int8 * MAX_TAPS) * MAX_PHASES),
+        ("tap_dw", (ctypes.c_int8 * MAX_TAPS) * MAX_PHASES),
+        ("workspace", c_ptr), ("splits", ctypes.c_int32),
+    ]
 
 
 # name -> (restype, argtypes); mirrors include/ipr_b200.h one to one (tests/test_abi.py checks it).
@@ -55,12 +88,12 @@ SIGNATURES = {
     "ipr_pdq_dct_matrix_host": (None, [c_ptr]),
     "ipr_pdq_hash_f32": (c_int, [c_ptr, c_ptr, c_ptr, c_ptr, c_i64, c_int, c_int, c_ptr]),
     "ipr_hash_pvalue": (c_int, [c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_i64, c_ptr]),
-    "ipr_tapgemm_m_tiles": (c_int, [c_ptr]),
-    "ipr_tapgemm_stats_rows": (c_int, [c_ptr]),
-    "ipr_tapgemm_bf16": (c_int, [c_ptr, c_ptr]),
-    "ipr_wgrad_workspace_bytes": (c_size, [c_ptr]),
-    "ipr_wgrad_total_kblocks": (c_int, [c_ptr]),
-    "ipr_wgrad_bf16": (c_int, [c_ptr, c_ptr]),
+    "ipr_tapgemm_m_tiles": (c_int, [ctypes.POINTER(TapGemm)]),
+    "ipr_tapgemm_stats_rows": (c_int, [ctypes.POINTER(TapGemm)]),
+    "ipr_tapgemm_bf16": (c_int, [ctypes.POINTER(TapGemm), c_ptr]),
+    "ipr_wgrad_workspace_bytes": (c_size, [ctypes.POINTER(WGrad)]),
+    "ipr_wgrad_total_kblocks": (c_int, [ctypes.POINTER(WGrad)]),
+    "ipr_wgrad_bf16": (c_int, [ctypes.POINTER(WGrad), c_ptr]),
     "ipr_im2col3_bf16": (c_int, [c_ptr, c_ptr, c_ptr, c_i64, c_int, c_int, c_ptr]),
     "ipr_col2im3_f32": (c_int, [c_ptr, c_ptr, c_i64, c_int, c_int, c_int, c_int, c_ptr]),
     "ipr_tapfold3_f32": (c_int, [c_ptr, c_ptr, c_ptr, c_ptr, c_i64, c_int, c_int, c_int, c_ptr]),
@@ -96,7 +129,7 @@ SIGNATURES = {
     "ipr_pointwise_loss_workspace_bytes": (c_size, []),
     "ipr_pointwise_loss_f32": (c_int, [c_ptr, c_ptr, c_f32, c_i64, c_int, c_f32, c_ptr, c_ptr, c_ptr, c_size, c_ptr]),
     "ipr_randn_f32": (c_int, [c_ptr, c_i64, ctypes.c_uint64, c_ptr, c_ptr, c_ptr]),
-    "ipr_wgrad_tiles": (c_int, [c_ptr]),
+    "ipr_wgrad_tiles": (c_int, [ctypes.POINTER(WGrad)]),
     "ipr_wgrad_reduce_f32": (c_int, [c_ptr, c_int, c_int, c_int, c_int, c_ptr, c_ptr, c_i64, c_ptr, c_int, c_f32, c_ptr]),
     "ipr_wgrad_reduce_taps_f32": (c_int, [c_ptr, c_int, c_int, c_int, c_int, c_int, c_ptr, c_int, c_i64, c_i64, c_ptr, c_int,
                                           ctypes.c_float, c_ptr]),

@@ -20,7 +20,6 @@
 //   tiles (6-8 smem stages, ~190 KB).
 #include "ipr_common.cuh"
 #include "tc_common.cuh"
-#include <stdlib.h>
 
 namespace {
 
@@ -53,8 +52,6 @@ struct TgParams {
     int8_t out_oh[IPR_TG_MAX_PHASES], out_ow[IPR_TG_MAX_PHASES];
     int n_valid;
     float *stats;
-    long long *dbg;        // optional phase timestamps of CTA 0 (scripts/tile_phase_probe.py)
-    int dbg_flags;         // probes only (IPR_TG_DBG_FLAGS): 1 = skip the output stores, 2 = skip the bias / activation math
 };
 
 __device__ __forceinline__ uint32_t pack_bf16x2(float lo, float hi) {
@@ -62,38 +59,29 @@ __device__ __forceinline__ uint32_t pack_bf16x2(float lo, float hi) {
     return *reinterpret_cast<uint32_t *>(&v);
 }
 
-// OCC = 2: two CTAs per SM for layers whose tiles have a short main loop (few k-blocks): there the epilogue -- one
-// warp per 32 rows walking its columns at ~0.2 instructions per cycle, ~2000 cycles per 128 x 64 tile (per-tile
-// timestamps, scripts/tile_phase_probe3.py) -- is the pace maker, and a second CTA doubles the epilogue warps per SM.
-// To fit, the variant keeps 3 smem stages, drains the accumulator 16 columns at a time (half the live registers:
-// <= 102 per thread) and stores rows directly.
 // TG = 2 ("tile groups"): the 8 epilogue warps form two groups of four that drain ALTERNATE tiles, each group with its
 // own pair of TMEM accumulators (4 in all).  A 128 x 64 tile has a main loop of a few hundred cycles but its read-out
 // (tcgen05.ld of 32 KB, then bias / activation / pack / store at ~0.4 instructions per cycle and scheduler) takes
-// ~1 900 (scripts/tile_phase_probe3.py); with all eight warps on the SAME tile the TMEM read-out and the arithmetic run
+// ~1 900 (per-tile clock64 stamps); with all eight warps on the SAME tile the TMEM read-out and the arithmetic run
 // strictly one after the other.  Two groups on different tiles overlap one group's tcgen05.ld with the other's math.
 // EPI / ST: the epilogue mode and "column statistics wanted" as COMPILE-TIME values for the hot combinations (-1 = read
 // them from the launch parameters).  The generic epilogue executes ~430 instructions per 32-column chunk, most of them
 // mode dispatch, register moves for the paths not taken and their address arithmetic (ncu source view, profiles/
 // r2_linear_case_generic_epilogue_full.txt); the low-K layers are paced by exactly that instruction stream.
-template <int BLOCK_N, int STAGES, int MT, bool RES, int EPI_WARPS, int OCC = 1, int TG = 1, int EPI = -1, int ST = -1>
-__global__ void __launch_bounds__(64 + EPI_WARPS * 32, OCC)
+template <int BLOCK_N, int STAGES, bool RES, int EPI_WARPS, int TG = 1, int EPI = -1, int ST = -1>
+__global__ void __launch_bounds__(64 + EPI_WARPS * 32, 1)
 tapgemm_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant__ CUtensorMap mapA1,
                const __grid_constant__ CUtensorMap mapA2, const __grid_constant__ CUtensorMap mapA3,
                const __grid_constant__ CUtensorMap mapB, const TgParams p)
 {
     constexpr int B_STAGE_BYTES = BLOCK_N * BLOCK_K * 2;
-    // MT = 2: the CTA tile is two 128-row sub-tiles that share ONE B (weight) tile in shared memory -- 1.36x more
-    // flops per byte streamed from L2, which is what bounds this kernel (about 10 TB/s L2->SM chip-wide)
-    constexpr int A_BYTES = MT * A_STAGE_BYTES;
-    constexpr int STAGE_BYTES = A_BYTES + B_STAGE_BYTES;
+    constexpr int STAGE_BYTES = A_STAGE_BYTES + B_STAGE_BYTES;
     constexpr uint32_t ACC_COLS = BLOCK_N < 32 ? 32 : BLOCK_N;     // TMEM columns of one accumulator
-    constexpr uint32_t BUF_COLS = MT * ACC_COLS;
     constexpr int NBUF = 2 * TG;                                     // accumulators in flight (two per tile group)
-    constexpr uint32_t TMEM_COLS = NBUF * BUF_COLS;                  // multi-buffered: epilogue(i) overlaps mainloop(i+1..)
+    constexpr uint32_t TMEM_COLS = NBUF * ACC_COLS;                  // multi-buffered: epilogue(i) overlaps mainloop(i+1..)
     static_assert(TMEM_COLS <= 512, "TMEM budget");
-    static_assert(TG == 1 || (EPI_WARPS == 8 && TG == 2 && MT == 1), "tile groups: two groups of four warps");
-    constexpr int CH = (BLOCK_N >= 32 && OCC == 1) ? 32 : 16;        // columns per tcgen05.ld
+    static_assert(TG == 1 || (EPI_WARPS == 8 && TG == 2), "tile groups: two groups of four warps");
+    constexpr int CH = BLOCK_N >= 32 ? 32 : 16;                      // columns per tcgen05.ld
     constexpr int N_CHUNKS = BLOCK_N / CH;
     constexpr int WARP_TMA = EPI_WARPS, WARP_MMA = EPI_WARPS + 1;
     constexpr int WPG = EPI_WARPS / TG;                              // warps per tile group
@@ -105,7 +93,7 @@ tapgemm_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
     extern __shared__ uint8_t smem_raw[];
     const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;     // SWIZZLE_128B needs 1024-byte alignment
     const uint32_t sA = smem_base;
-    const uint32_t sB = smem_base + STAGES * A_BYTES;
+    const uint32_t sB = smem_base + STAGES * A_STAGE_BYTES;
     // RES: the whole weight matrix of this layer (all taps, all phases; one N block) stays resident in shared memory
     // for the lifetime of the persistent CTA, so only A tiles are streamed -- the kernel is paced by TMA row requests
     // (128 A rows + BLOCK_N B rows per k-block), and high-resolution layers have small weights
@@ -119,19 +107,14 @@ tapgemm_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
     const uint32_t tmem_slot = bar_bres + 8;
 
     // per-warp running column statistics [epilogue warp][sum | sumsq][CH_PER_WARP * CH] floats (after the mbarriers)
-    float *stat_sm = reinterpret_cast<float *>(smem_raw + (smem_base - smem_u32(smem_raw)) + STAGES * A_BYTES + b_region + 256);
+    float *stat_sm = reinterpret_cast<float *>(smem_raw + (smem_base - smem_u32(smem_raw)) + STAGES * A_STAGE_BYTES + b_region + 256);
     // per-epilogue-warp staging (2 KB each) for the transposed bf16 store: behind the statistics slots, 16-byte aligned
     uint8_t *stage_sm = reinterpret_cast<uint8_t *>(stat_sm) + TG * 8 * BLOCK_N * 4;
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    if (p.dbg && threadIdx.x == 0) {
-        unsigned long long gt; asm volatile("mov.u64 %0, %globaltimer;" : "=l"(gt));
-        p.dbg[64 + blockIdx.x * 2] = (long long)gt;
-    }
     const int num_kb = p.n_taps * p.c_chunks;
     const int n_blks = p.n_total / BLOCK_N;
-    const int m_groups = (p.m_tiles + MT - 1) / MT;                 // CTA tiles along M
-    const int tiles_per_phase = m_groups * n_blks;
+    const int tiles_per_phase = p.m_tiles * n_blks;
     const int total_tiles = tiles_per_phase * p.n_phases;
 
     if (warp == WARP_TMA && lane == 0) {
@@ -164,26 +147,20 @@ tapgemm_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
             }
             for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x) {
                 const int phase = tile / tiles_per_phase, rem = tile - phase * tiles_per_phase;
-                const int m_grp = rem / n_blks, n_blk = rem - m_grp * n_blks;
-                int img0[MT], h0[MT];
-#pragma unroll
-                for (int j = 0; j < MT; j++) {
-                    const int m_tile = m_grp * MT + j;              // a tile past the end reads zeros (TMA out-of-bounds fill)
-                    if (p.tile_imgs == 1) { img0[j] = m_tile / p.tiles_per_img; h0[j] = (m_tile - img0[j] * p.tiles_per_img) * p.tile_h; }
-                    else { img0[j] = m_tile * p.tile_imgs; h0[j] = 0; }
-                }
+                const int m_tile = rem / n_blks, n_blk = rem - m_tile * n_blks;
+                int img0, h0;
+                if (p.tile_imgs == 1) { img0 = m_tile / p.tiles_per_img; h0 = (m_tile - img0 * p.tiles_per_img) * p.tile_h; }
+                else { img0 = m_tile * p.tile_imgs; h0 = 0; }
                 for (int kb = 0; kb < num_kb; kb++, g++) {
                     const int s = g % STAGES;
                     const uint32_t par = (g / STAGES) & 1u;
                     mbar_wait(bar_empty + 8 * s, par ^ 1u);
-                    mbar_expect_tx(bar_full + 8 * s, RES ? A_BYTES : STAGE_BYTES);
+                    mbar_expect_tx(bar_full + 8 * s, RES ? A_STAGE_BYTES : STAGE_BYTES);
                     const int tap = kb / p.c_chunks, cc = kb - tap * p.c_chunks;
                     const int mi = p.tap_map[phase][tap];
                     const CUtensorMap *ma = mi == 0 ? &mapA0 : (mi == 1 ? &mapA1 : (mi == 2 ? &mapA2 : &mapA3));
-#pragma unroll
-                    for (int j = 0; j < MT; j++)
-                        tma_load_4d(sA + s * A_BYTES + j * A_STAGE_BYTES, ma, bar_full + 8 * s, cc * BLOCK_K,
-                                    (int)p.tap_dw[phase][tap], h0[j] + (int)p.tap_dh[phase][tap], img0[j]);
+                    tma_load_4d(sA + s * A_STAGE_BYTES, ma, bar_full + 8 * s, cc * BLOCK_K, (int)p.tap_dw[phase][tap],
+                                h0 + (int)p.tap_dh[phase][tap], img0);
                     if (!RES)
                         tma_load_2d(sB + s * B_STAGE_BYTES, &mapB, bar_full + 8 * s, tap * p.a_c + cc * BLOCK_K,
                                     phase * p.n_total + n_blk * BLOCK_N);
@@ -200,32 +177,24 @@ tapgemm_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
             for (int tile = blockIdx.x; tile < total_tiles; tile += gridDim.x, it++) {
                 const int phase_m = tile / tiles_per_phase;
                 const uint32_t buf = it % NBUF;
-                if (p.dbg && blockIdx.x == 0 && it < 8) p.dbg[it * 8 + 0] = clock64();
                 mbar_wait(bar_acc_empty + 8 * buf, ((it / NBUF) & 1u) ^ 1u);    // epilogue drained this accumulator
-                if (p.dbg && blockIdx.x == 0 && it < 8) p.dbg[it * 8 + 1] = clock64();
                 tc_fence_after();
-                const uint32_t acc = tmem_base + buf * BUF_COLS;
+                const uint32_t acc = tmem_base + buf * ACC_COLS;
                 for (int kb = 0; kb < num_kb; kb++, g++) {
                     const int s = g % STAGES;
                     const uint32_t par = (g / STAGES) & 1u;
                     mbar_wait(bar_full + 8 * s, par);
                     tc_fence_after();
+                    const uint64_t da = umma_desc_sw128(sA + s * A_STAGE_BYTES, 0, 1024);
                     const uint64_t db = umma_desc_sw128(RES ? sB + (phase_m * num_kb + kb) * B_STAGE_BYTES
                                                             : sB + s * B_STAGE_BYTES, 0, 1024);
+                    // advance 32 bytes (16 bf16) along K inside the swizzle atom: +2 in the (addr >> 4) field
 #pragma unroll
-                    for (int k = 0; k < BLOCK_K / UMMA_K; k++) {
-#pragma unroll
-                        for (int j = 0; j < MT; j++) {
-                            // advance 32 bytes (16 bf16) along K inside the swizzle atom: +2 in the (addr >> 4) field
-                            const uint64_t da = umma_desc_sw128(sA + s * A_BYTES + j * A_STAGE_BYTES, 0, 1024);
-                            umma_bf16(acc + j * ACC_COLS, da + (uint64_t)(2 * k), db + (uint64_t)(2 * k), idesc,
-                                      (kb | k) != 0 ? 1u : 0u);
-                        }
-                    }
+                    for (int k = 0; k < BLOCK_K / UMMA_K; k++)
+                        umma_bf16(acc, da + (uint64_t)(2 * k), db + (uint64_t)(2 * k), idesc, (kb | k) != 0 ? 1u : 0u);
                     umma_commit(bar_empty + 8 * s);           // smem stage reusable once these MMAs retire
                 }
                 umma_commit(bar_acc_full + 8 * buf);          // accumulator complete
-                if (p.dbg && blockIdx.x == 0 && it < 8) p.dbg[it * 8 + 2] = clock64();
             }
         }
         __syncwarp();
@@ -241,46 +210,45 @@ tapgemm_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
         const float inv_sigma = p.sigma ? 1.0f / __ldg(p.sigma) : 1.0f;
         // EPI_MASK reads one activation row per thread and chunk.  Those loads miss to L2/HBM (~1 us): issued after
         // the accumulator wait they serialise every chunk behind a full memory round trip.  A walker therefore runs two
-        // chunks ahead of the (tile, sub, chunk) sequence and keeps their mask words in a register FIFO, so the loads
+        // chunks ahead of the (tile, chunk) sequence and keeps their mask words in a register FIFO, so the loads
         // for the next tile are in flight while this warp still waits for that tile's MMAs.
         constexpr int MQ = CH / 8;                         // uint4 per thread and chunk
         uint4 mq0[MQ], mq1[MQ];
-        // Tile coordinates advance by gridDim.x every iteration: (phase, m_grp, n_blk) are stepped incrementally and the
+        // Tile coordinates advance by gridDim.x every iteration: (phase, m_tile, n_blk) are stepped incrementally and the
         // pixel of a row is (per-tile uniform part) + (per-thread constant part) -- no division in the tile loop.
         const int t_step = TG * (int)gridDim.x;           // a group's next tile
         const int g_q = t_step / n_blks, g_r = t_step - g_q * n_blks;
         const int tpi_shift = (p.tiles_per_img & (p.tiles_per_img - 1)) == 0 ? 31 - __clz(p.tiles_per_img) : -1;
         const int thr_pix = (i_img * p.out_h + i_row * p.out_sh) * p.out_w + i_col * p.out_sw;
-        struct TileIt { int tile, phase, m_grp, n_blk; };
+        struct TileIt { int tile, phase, m_tile, n_blk; };
         auto it_init = [&](TileIt &t) {
             t.tile = blockIdx.x + grp * gridDim.x;
             t.phase = t.tile / tiles_per_phase;
             const int rm = t.tile - t.phase * tiles_per_phase;
-            t.m_grp = rm / n_blks; t.n_blk = rm - t.m_grp * n_blks;
+            t.m_tile = rm / n_blks; t.n_blk = rm - t.m_tile * n_blks;
         };
         auto it_next = [&](TileIt &t) {
-            t.tile += t_step; t.n_blk += g_r; t.m_grp += g_q;
-            if (t.n_blk >= n_blks) { t.n_blk -= n_blks; t.m_grp++; }
-            while (t.m_grp >= m_groups) { t.m_grp -= m_groups; t.phase++; }
+            t.tile += t_step; t.n_blk += g_r; t.m_tile += g_q;
+            if (t.n_blk >= n_blks) { t.n_blk -= n_blks; t.m_tile++; }
+            while (t.m_tile >= p.m_tiles) { t.m_tile -= p.m_tiles; t.phase++; }
         };
-        // -> pixel index of this thread's row in tile (t, sub), or -1 when the row is outside the tensor
-        auto row_pix = [&](const TileIt &t, int sub) -> long long {
-            const int mt = t.m_grp * MT + sub;
+        // -> pixel index of this thread's row in tile t, or -1 when the row is outside the tensor
+        auto row_pix = [&](const TileIt &t) -> long long {
             int im0, hh0;
             if (p.tile_imgs == 1) {
-                im0 = tpi_shift >= 0 ? (mt >> tpi_shift) : mt / p.tiles_per_img;
-                hh0 = (mt - im0 * p.tiles_per_img) * p.tile_h;
-            } else { im0 = mt * p.tile_imgs; hh0 = 0; }
-            if (!(im0 + i_img < p.a_n && mt < p.m_tiles)) return -1;
+                im0 = tpi_shift >= 0 ? (t.m_tile >> tpi_shift) : t.m_tile / p.tiles_per_img;
+                hh0 = (t.m_tile - im0 * p.tiles_per_img) * p.tile_h;
+            } else { im0 = t.m_tile * p.tile_imgs; hh0 = 0; }
+            if (im0 + i_img >= p.a_n) return -1;
             return (long long)(im0 * p.out_h + hh0 * p.out_sh + p.out_oh[t.phase]) * p.out_w + p.out_ow[t.phase] + thr_pix;
         };
         TileIt wt;                                         // the walker's position
-        int w_sub = 0, w_c0 = c_begin;
-        const __nv_bfloat16 *w_base = nullptr;             // mask row of the walker's (tile, sub), nullptr when masked out
+        int w_c0 = c_begin;
+        const __nv_bfloat16 *w_base = nullptr;             // mask row of the walker's tile, nullptr when masked out
         auto w_locate = [&]() {
             w_base = nullptr;
             if (wt.tile >= total_tiles) return;
-            const long long px = row_pix(wt, w_sub);
+            const long long px = row_pix(wt);
             if (px >= 0) w_base = p.mask + px * p.out_c + wt.n_blk * BLOCK_N;
         };
         auto w_fetch = [&](uint4 (&dst)[MQ]) {
@@ -291,7 +259,7 @@ tapgemm_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
             w_c0 += CH;
             if (w_c0 >= c_end) {
                 w_c0 = c_begin;
-                if (++w_sub >= MT) { w_sub = 0; it_next(wt); }
+                it_next(wt);
                 w_locate();
             }
         };
@@ -314,9 +282,8 @@ tapgemm_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
         TileIt ct;
         it_init(ct);
         for (; ct.tile < total_tiles; it_next(ct), it += TG) {
-            const int phase = ct.phase, m_grp = ct.m_grp, n_blk = ct.n_blk;
+            const int phase = ct.phase, m_tile = ct.m_tile, n_blk = ct.n_blk;
             const uint32_t buf = it % NBUF;
-            if (p.dbg && blockIdx.x == 0 && it < 8 && warp == 0 && lane == 0) p.dbg[it * 8 + 3] = clock64();
             // bias (and eval-BatchNorm scale) of the tile's FIRST chunk: fetched before the accumulator wait, so the loads
             // are in flight while the main loop of this tile still runs (they used to stall the first FADDs)
             constexpr bool PRE = EPI == IPR_EPI_BIAS_LRELU;     // only where the mode is known at compile time (registers)
@@ -332,12 +299,8 @@ tapgemm_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
             }
             mbar_wait_backoff(bar_acc_full + 8 * buf, (it / NBUF) & 1u);
             tc_fence_after();
-            if (p.dbg && blockIdx.x == 0 && it < 8 && warp == 0 && lane == 0) p.dbg[it * 8 + 4] = clock64();
-#pragma unroll 1
-          for (int sub = 0; sub < MT; sub++) {
-            const int m_tile = m_grp * MT + sub;
-            const long long pix_s = row_pix(ct, sub);
-            const bool valid = pix_s >= 0 && !(p.dbg_flags & 1);
+            const long long pix_s = row_pix(ct);
+            const bool valid = pix_s >= 0;
             const size_t pix = (size_t)pix_s;
 #pragma unroll 1
             for (int c0 = c_begin; c0 < c_end; c0 += CH) {
@@ -348,11 +311,11 @@ tapgemm_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
                     for (int g = 0; g < MQ; g++) { mcur[g] = mq0[g]; mq0[g] = mq1[g]; }
                     w_fetch(mq1);
                 }
-                const uint32_t taddr = tmem_base + buf * BUF_COLS + sub * ACC_COLS + ((uint32_t)(q * 32) << 16) + (uint32_t)c0;
+                const uint32_t taddr = tmem_base + buf * ACC_COLS + ((uint32_t)(q * 32) << 16) + (uint32_t)c0;
                 if constexpr (CH == 32) tmem_ld_32x32(taddr, raw);
                 else tmem_ld_32x16(taddr, *reinterpret_cast<uint32_t(*)[16]>(&raw));
                 tmem_ld_wait();
-                if (c0 + CH >= c_end && sub == MT - 1) {
+                if (c0 + CH >= c_end) {
                     // last chunk is in registers: hand the accumulator back to the MMA warp before the slow part
                     tc_fence_before();
                     __syncwarp();
@@ -367,8 +330,8 @@ tapgemm_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
                     for (int j = 0; j < CH; j++) v[j] *= inv_sigma;
                 }
 
-                if (epi_mode == IPR_EPI_BIAS_LRELU && !(p.dbg_flags & 2)) {
-                    const bool first = pre_bias && sub == 0 && c0 == c_begin;
+                if (epi_mode == IPR_EPI_BIAS_LRELU) {
+                    const bool first = pre_bias && c0 == c_begin;
                     if (p.scale) {                         // eval-mode BatchNorm folded into the layer: per-column factor
 #pragma unroll
                         for (int j4 = 0; j4 < CH / 4; j4++) {
@@ -484,8 +447,8 @@ tapgemm_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
                             // per-warp staging area (XOR-swizzled 16-byte slots: conflict-free both ways) one
                             // instruction writes 8 rows x 64 contiguous bytes: a quarter of the line touches.
                             // Measured: neutral for the step (patch GEMM 48.0 -> 46.6 us) -- disabling the stores
-                            // altogether changes nothing either (IPR_TG_DBG_FLAGS=1); the epilogue is paced by its
-                            // instruction stream, see the EPI / ST template parameters.
+                            // altogether changes nothing either; the epilogue is paced by its instruction stream, see
+                            // the EPI / ST template parameters.
                             uint8_t *stg = stage_sm + warp * 2048;
 #pragma unroll
                             for (int gq = 0; gq < 4; gq++)
@@ -512,8 +475,6 @@ tapgemm_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
                     }
                 }
             }
-          }
-          if (p.dbg && blockIdx.x == 0 && it < 8 && warp == 0 && lane == 0) p.dbg[it * 8 + 5] = clock64();
         }
         if (cta_stats) {
             __syncwarp();
@@ -527,99 +488,90 @@ tapgemm_kernel(const __grid_constant__ CUtensorMap mapA0, const __grid_constant_
     tc_fence_before();
     __syncthreads();
     if (warp == WARP_MMA) tmem_dealloc(tmem_base, TMEM_COLS);
-    if (p.dbg && threadIdx.x == 0) {
-        unsigned long long gt; asm volatile("mov.u64 %0, %globaltimer;" : "=l"(gt));
-        p.dbg[64 + blockIdx.x * 2 + 1] = (long long)gt;
-    }
 }
 
-template <int BLOCK_N, int STAGES, int MT, bool RES, int EW, int OCC = 1, int TG = 1, int EPI = -1, int ST = -1>
+template <int BLOCK_N, int STAGES, bool RES, int EW, int TG = 1, int EPI = -1, int ST = -1>
 int launch_ew(const CUtensorMap *ma, const CUtensorMap &mb, const TgParams &p, dim3 grid, cudaStream_t st)
 {
     const size_t b_region = RES ? (size_t)p.n_phases * p.n_taps * p.c_chunks * BLOCK_N * BLOCK_K * 2
                                 : (size_t)STAGES * BLOCK_N * BLOCK_K * 2;
-    const size_t smem = (size_t)STAGES * MT * A_STAGE_BYTES + b_region + 256 + TG * 8 * BLOCK_N * 4 + (OCC == 1 ? 8 * 2048 : 0) + 1024 + 64;
-    if (smem > (size_t)(OCC == 1 ? 227 : 113) * 1024) return IPR_E_UNSUPPORTED;
+    const size_t smem = (size_t)STAGES * A_STAGE_BYTES + b_region + 256 + TG * 8 * BLOCK_N * 4 + 8 * 2048 + 1024 + 64;
+    if (smem > (size_t)227 * 1024) return IPR_E_UNSUPPORTED;
     static bool attr = false;
     if (!attr) {
-        cudaError_t e = cudaFuncSetAttribute(tapgemm_kernel<BLOCK_N, STAGES, MT, RES, EW, OCC, TG, EPI, ST>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                             (OCC == 1 ? 227 : 113) * 1024);
+        cudaError_t e = cudaFuncSetAttribute(tapgemm_kernel<BLOCK_N, STAGES, RES, EW, TG, EPI, ST>,
+                                             cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
         if (e != cudaSuccess) return (int)e;
         attr = true;
     }
-    const int total = (int)(((grid.x + MT - 1) / MT) * grid.y * grid.z);
-    const int slots = ipr_sm_count() * OCC;                                  // persistent: OCC CTAs per SM
-    const int ctas = total < slots ? total : slots;
-    IPR_LAUNCH_PDL((tapgemm_kernel<BLOCK_N, STAGES, MT, RES, EW, OCC, TG, EPI, ST>), ctas, 64 + EW * 32, smem, st, ma[0], ma[1], ma[2], ma[3], mb, p);
+    const int total = (int)(grid.x * grid.y * grid.z);
+    const int ctas = total < ipr_sm_count() ? total : ipr_sm_count();       // persistent: one CTA per SM
+    IPR_LAUNCH_PDL((tapgemm_kernel<BLOCK_N, STAGES, RES, EW, TG, EPI, ST>), ctas, 64 + EW * 32, smem, st, ma[0], ma[1], ma[2], ma[3], mb, p);
     IPR_LAUNCH_CHECK();
     return IPR_OK;
 }
 
-// Two tile groups (TG = 2) where the epilogue does per-element work (the `wide` case below) and every CTA has at least
-// four tiles; same rule in ipr_tapgemm_stats_rows (the per-CTA statistics rows double).
-bool wide_epilogue(const TgParams &p)
-{
-    static const char *force = getenv("IPR_TG_EPI_WARPS");
-    const bool heavy = p.epi_mode == IPR_EPI_BIAS_LRELU || p.epi_mode == IPR_EPI_MASK || p.stats != nullptr;
-    return force ? force[0] == '8' : heavy;
-}
-bool use_tile_groups(const TgParams &p, int block_n, dim3 grid)
-{
-    static const char *off = getenv("IPR_TG_NO_GROUPS");
-    if (off) return false;
-    const long long tiles = (long long)grid.x * grid.y * grid.z;
-    // Measured (scripts/ab_groups.sh, batch 512): the single-k-block patch GEMM gains (32->64 bias+LeakyReLU 46.3 -> 40.6 us);
-    // layers with a real main loop do not (convT4s2 128->64 79 -> 82 us, conv3_dgrad 128->64 44.5 -> 46.6 us), so the
-    // groups are used for main loops of at most two k-blocks.
-    return block_n >= 32 && block_n <= 128 && tiles >= 4LL * ipr_sm_count() && p.n_taps * p.c_chunks <= 2;
-}
+// The kernel variant of one launch, chosen from the descriptor and the tile count alone: ipr_tapgemm_bf16 launches it
+// and ipr_tapgemm_stats_rows sizes the statistics from it.  The smem stages follow from BLOCK_N and RES (see launch).
+struct Variant {
+    bool resident;        // RES
+    int epi_warps;        // EW
+    int tile_groups;      // TG
+    int epi, stats;       // EPI, ST: -1 = the generic epilogue, which reads them from the launch parameters
+};
 
-// Two CTAs per SM pay off where a tile's main loop is shorter than its epilogue: few k-blocks per tile, enough tiles.
-bool use_two_ctas(const ipr_tapgemm_t *d, const TgParams &p)
+Variant pick_variant(const ipr_tapgemm_t *d, int m_tiles, bool stats)
 {
-    // Measured on B200 (scripts/ab_run.sh, batch 512): the variant LOSES -- patch GEMM 32->64 47 -> 69 us, conv4s2_dgrad
-    // 64->64 78 -> 112 us, step 4.05 -> 4.39 ms -- so it is opt-in (IPR_TG_OCC2=1) and kept only as a probe.
-    static const char *on = getenv("IPR_TG_OCC2");
-    if (!on) return false;
     const int num_kb = d->n_taps * ((d->a_c + BLOCK_K - 1) / BLOCK_K);
-    const long long tiles = (long long)p.m_tiles * (d->n_total / d->block_n) * d->n_phases;
-    const int kb_limit = d->block_n == 64 ? 10 : 5;                          // main loop <= ~1300 cycles
-    return (d->block_n == 64 || d->block_n == 128) && num_kb <= kb_limit && tiles >= 4LL * ipr_sm_count() &&
-           d->epi_mode != IPR_EPI_TANH_NCHW && d->epi_mode != IPR_EPI_LINEAR_NCHW;
+    const long long tiles = (long long)m_tiles * (d->n_total / d->block_n) * d->n_phases;
+    const long long sms = ipr_sm_count();
+    Variant v;
+    // weights resident in shared memory: one N block, everything (all phases x taps) fits beside 4 A stages, and every
+    // CTA has at least two tiles to amortise the one-off weight load over
+    const size_t b_all = (size_t)d->n_phases * num_kb * d->block_n * BLOCK_K * 2;
+    v.resident = d->block_n <= 128 && d->n_total == d->block_n && b_all <= 132 * 1024 && tiles >= 2 * sms;
+    const bool heavy = d->epi_mode == IPR_EPI_BIAS_LRELU || d->epi_mode == IPR_EPI_MASK || stats;
+    v.epi_warps = heavy ? 8 : 4;
+    v.tile_groups = 1;
+    v.epi = v.stats = -1;
+    if (!heavy) {
+        if (d->epi_mode == IPR_EPI_LINEAR || d->epi_mode == IPR_EPI_LINEAR_F32) { v.epi = d->epi_mode; v.stats = 0; }
+        return v;
+    }
+    if (d->epi_mode == IPR_EPI_BIAS_LRELU && !stats) { v.epi = IPR_EPI_BIAS_LRELU; v.stats = 0; }
+    else if (d->epi_mode == IPR_EPI_MASK) { v.epi = IPR_EPI_MASK; v.stats = stats ? 1 : 0; }
+    else if (d->epi_mode == IPR_EPI_LINEAR && stats) { v.epi = IPR_EPI_LINEAR; v.stats = 1; }
+    // Two tile groups need every CTA to have at least four tiles.  Measured (batch 512): the single-k-block patch GEMM
+    // gains (32->64 bias+LeakyReLU 46.3 -> 40.6 us); layers with a real main loop do not (convT4s2 128->64 79 -> 82 us,
+    // conv3_dgrad 128->64 44.5 -> 46.6 us), so the groups are used for main loops of at most two k-blocks.  Of the
+    // specialised epilogues only bias + LeakyReLU has a tile-group version.
+    if ((v.epi == -1 || v.epi == IPR_EPI_BIAS_LRELU) && d->block_n >= 32 && d->block_n <= 128 && tiles >= 4 * sms &&
+        num_kb <= 2)
+        v.tile_groups = 2;
+    return v;
 }
 
-template <int BLOCK_N, int STAGES, int MT, bool RES>
-int launch(const CUtensorMap *ma, const CUtensorMap &mb, const TgParams &p, dim3 grid, cudaStream_t st)
+template <int BLOCK_N, bool RES>
+int launch(const Variant &v, const CUtensorMap *ma, const CUtensorMap &mb, const TgParams &p, dim3 grid, cudaStream_t st)
 {
-    const bool wide = wide_epilogue(p);
-    if (MT == 1 && wide) {
-        static const char *generic = getenv("IPR_TG_GENERIC_EPI");
-        const bool stats = p.stats != nullptr;
-        if (!generic) {
-            if (p.epi_mode == IPR_EPI_BIAS_LRELU && !stats) {
-                if constexpr (BLOCK_N >= 32 && BLOCK_N <= 128) {
-                    if (use_tile_groups(p, BLOCK_N, grid))
-                        return launch_ew<BLOCK_N, STAGES, 1, RES, 8, 1, 2, IPR_EPI_BIAS_LRELU, 0>(ma, mb, p, grid, st);
-                }
-                return launch_ew<BLOCK_N, STAGES, 1, RES, 8, 1, 1, IPR_EPI_BIAS_LRELU, 0>(ma, mb, p, grid, st);
-            }
-            if (p.epi_mode == IPR_EPI_MASK)
-                return stats ? launch_ew<BLOCK_N, STAGES, 1, RES, 8, 1, 1, IPR_EPI_MASK, 1>(ma, mb, p, grid, st)
-                             : launch_ew<BLOCK_N, STAGES, 1, RES, 8, 1, 1, IPR_EPI_MASK, 0>(ma, mb, p, grid, st);
-            if (p.epi_mode == IPR_EPI_LINEAR && stats)
-                return launch_ew<BLOCK_N, STAGES, 1, RES, 8, 1, 1, IPR_EPI_LINEAR, 1>(ma, mb, p, grid, st);
-        }
-        if constexpr (BLOCK_N >= 32 && BLOCK_N <= 128) {
-            if (use_tile_groups(p, BLOCK_N, grid)) return launch_ew<BLOCK_N, STAGES, 1, RES, 8, 1, 2>(ma, mb, p, grid, st);
-        }
-        return launch_ew<BLOCK_N, STAGES, 1, RES, 8>(ma, mb, p, grid, st);
+    // smem stages: 4 A stages beside a resident weight matrix, otherwise as many A + B stages as fit in ~190 KB
+    constexpr int S = RES ? 4 : (BLOCK_N <= 64 ? 8 : (BLOCK_N == 128 ? 6 : 4));
+    if (v.epi_warps == 4) {
+        if (v.epi == IPR_EPI_LINEAR) return launch_ew<BLOCK_N, S, RES, 4, 1, IPR_EPI_LINEAR, 0>(ma, mb, p, grid, st);
+        if (v.epi == IPR_EPI_LINEAR_F32) return launch_ew<BLOCK_N, S, RES, 4, 1, IPR_EPI_LINEAR_F32, 0>(ma, mb, p, grid, st);
+        return launch_ew<BLOCK_N, S, RES, 4>(ma, mb, p, grid, st);
     }
-    static const char *generic_light = getenv("IPR_TG_GENERIC_EPI");
-    if (MT == 1 && p.stats == nullptr && generic_light == nullptr) {       // the light (4-warp) combinations
-        if (p.epi_mode == IPR_EPI_LINEAR) return launch_ew<BLOCK_N, STAGES, 1, RES, 4, 1, 1, IPR_EPI_LINEAR, 0>(ma, mb, p, grid, st);
-        if (p.epi_mode == IPR_EPI_LINEAR_F32) return launch_ew<BLOCK_N, STAGES, 1, RES, 4, 1, 1, IPR_EPI_LINEAR_F32, 0>(ma, mb, p, grid, st);
+    if constexpr (BLOCK_N >= 32 && BLOCK_N <= 128) {
+        if (v.tile_groups == 2)
+            return v.epi == IPR_EPI_BIAS_LRELU ? launch_ew<BLOCK_N, S, RES, 8, 2, IPR_EPI_BIAS_LRELU, 0>(ma, mb, p, grid, st)
+                                               : launch_ew<BLOCK_N, S, RES, 8, 2>(ma, mb, p, grid, st);
     }
-    return launch_ew<BLOCK_N, STAGES, MT, RES, 4>(ma, mb, p, grid, st);
+    if (v.epi == IPR_EPI_BIAS_LRELU) return launch_ew<BLOCK_N, S, RES, 8, 1, IPR_EPI_BIAS_LRELU, 0>(ma, mb, p, grid, st);
+    if (v.epi == IPR_EPI_MASK)
+        return v.stats ? launch_ew<BLOCK_N, S, RES, 8, 1, IPR_EPI_MASK, 1>(ma, mb, p, grid, st)
+                       : launch_ew<BLOCK_N, S, RES, 8, 1, IPR_EPI_MASK, 0>(ma, mb, p, grid, st);
+    if (v.epi == IPR_EPI_LINEAR) return launch_ew<BLOCK_N, S, RES, 8, 1, IPR_EPI_LINEAR, 1>(ma, mb, p, grid, st);
+    return launch_ew<BLOCK_N, S, RES, 8>(ma, mb, p, grid, st);
 }
 
 int tile_geometry(const ipr_tapgemm_t *d, TgParams &p)
@@ -653,12 +605,10 @@ extern "C" int ipr_tapgemm_stats_rows(const ipr_tapgemm_t *d)
     if (rc != IPR_OK) return rc;
     IPR_REQUIRE(d->block_n > 0 && d->n_total % d->block_n == 0 && d->n_phases >= 1, IPR_E_SHAPE);
     const long long tiles = (long long)p.m_tiles * d->n_phases;
-    p.n_taps = d->n_taps; p.c_chunks = (d->a_c + BLOCK_K - 1) / BLOCK_K;
-    const long long slots = (long long)ipr_sm_count() * (use_two_ctas(d, p) ? 2 : 1);
-    // statistics imply the wide (8-warp) epilogue; with two tile groups every CTA writes 4 rows per group
-    const bool groups = !use_two_ctas(d, p) && use_tile_groups(p, d->block_n, dim3((unsigned)p.m_tiles, 1, (unsigned)d->n_phases));
-    if (d->n_total == d->block_n) return (int)(4 * (groups ? 2 : 1) * (tiles < slots ? tiles : slots));
-    return (int)(4 * tiles);
+    if (d->n_total != d->block_n) return (int)(4 * tiles);          // 4 rows per tile
+    // one N block: 4 rows per CTA and tile group
+    const long long ctas = tiles < ipr_sm_count() ? tiles : ipr_sm_count();
+    return (int)(4 * pick_variant(d, p.m_tiles, true).tile_groups * ctas);
 }
 
 extern "C" int ipr_tapgemm_m_tiles(const ipr_tapgemm_t *d)
@@ -708,11 +658,6 @@ extern "C" int ipr_tapgemm_bf16(const ipr_tapgemm_t *d, ipr_stream_t stream)
     p.mask = (const __nv_bfloat16 *)d->mask; p.out = d->out;
     p.out_h = d->out_h; p.out_w = d->out_w; p.out_c = d->out_c; p.out_sh = d->out_sh; p.out_sw = d->out_sw;
     p.n_valid = d->n_valid > 0 ? d->n_valid : d->n_total; p.stats = d->stats;
-    // probe switches are read ONCE per process (every getenv walks the whole environment: ~0.5 us each, five per launch)
-    static const char *dbg_ptr = getenv("IPR_TG_DBG_PTR"), *dbg_flags = getenv("IPR_TG_DBG_FLAGS");
-    static const char *env_pair = getenv("IPR_TG_PAIR"), *env_no_res = getenv("IPR_TG_NO_RESIDENT");
-    p.dbg = dbg_ptr ? (long long *)strtoull(dbg_ptr, nullptr, 0) : nullptr;
-    p.dbg_flags = dbg_flags ? atoi(dbg_flags) : 0;
 
     // ---- tensor maps (host-encoded, passed by value as kernel parameters: graph-capturable)
     CUtensorMap ma[4], mb;
@@ -746,36 +691,12 @@ extern "C" int ipr_tapgemm_bf16(const ipr_tapgemm_t *d, ipr_stream_t stream)
     }
     dim3 grid((unsigned)p.m_tiles, (unsigned)(d->n_total / d->block_n), (unsigned)d->n_phases);
     cudaStream_t st = ipr_cu(stream);
-    // Two M sub-tiles per CTA sharing one weight tile (25 % fewer bytes per flop) is implemented but OFF by default:
-    // on B200 it measured no faster (conv3 64->128 @16, batch 512: 590 vs 650 TFLOP/s; step 5.08 vs 5.02 ms) -- with
-    // the same 192 KB in flight the per-SM TMA throughput dropped from ~35 to ~24 B/clk.  IPR_TG_PAIR=1 enables it.
-    const long long single_tiles = (long long)grid.x * grid.y * grid.z;
-    const bool pair = single_tiles >= 3LL * ipr_sm_count() && env_pair != nullptr && !d->stats;   // stats rows assume MT = 1
-    // weights resident in shared memory: one N block, everything (all phases x taps) fits beside 4 A stages, and every
-    // CTA has at least two tiles to amortise the one-off weight load over
-    const size_t b_all = (size_t)d->n_phases * d->n_taps * p.c_chunks * d->block_n * BLOCK_K * 2;
-    const bool resident = d->n_total == d->block_n && b_all <= 132 * 1024 && single_tiles >= 2LL * ipr_sm_count() &&
-                          env_no_res == nullptr;
-    if (!pair && use_two_ctas(d, p)) {
-        const bool heavy = p.epi_mode == IPR_EPI_BIAS_LRELU || p.epi_mode == IPR_EPI_MASK || p.stats != nullptr;
-        (void)heavy;
-        if (d->block_n == 64) return launch_ew<64, 3, 1, false, 8, 2>(ma, mb, p, grid, st);
-        return launch_ew<128, 3, 1, false, 8, 2>(ma, mb, p, grid, st);
-    }
-    if (resident) {
-        switch (d->block_n) {
-            case 16:  return launch<16, 4, 1, true>(ma, mb, p, grid, st);
-            case 32:  return launch<32, 4, 1, true>(ma, mb, p, grid, st);
-            case 64:  return launch<64, 4, 1, true>(ma, mb, p, grid, st);
-            case 128: return launch<128, 4, 1, true>(ma, mb, p, grid, st);
-            default:  break;
-        }
-    }
+    const Variant v = pick_variant(d, p.m_tiles, d->stats != nullptr);
     switch (d->block_n) {
-        case 16:  return launch<16, 8, 1, false>(ma, mb, p, grid, st);
-        case 32:  return launch<32, 8, 1, false>(ma, mb, p, grid, st);
-        case 64:  return pair ? launch<64, 5, 2, false>(ma, mb, p, grid, st) : launch<64, 8, 1, false>(ma, mb, p, grid, st);
-        case 128: return pair ? launch<128, 4, 2, false>(ma, mb, p, grid, st) : launch<128, 6, 1, false>(ma, mb, p, grid, st);
-        default:  return launch<256, 4, 1, false>(ma, mb, p, grid, st);
+        case 16:  return v.resident ? launch<16, true>(v, ma, mb, p, grid, st) : launch<16, false>(v, ma, mb, p, grid, st);
+        case 32:  return v.resident ? launch<32, true>(v, ma, mb, p, grid, st) : launch<32, false>(v, ma, mb, p, grid, st);
+        case 64:  return v.resident ? launch<64, true>(v, ma, mb, p, grid, st) : launch<64, false>(v, ma, mb, p, grid, st);
+        case 128: return v.resident ? launch<128, true>(v, ma, mb, p, grid, st) : launch<128, false>(v, ma, mb, p, grid, st);
+        default:  return launch<256, false>(v, ma, mb, p, grid, st);
     }
 }

@@ -8,13 +8,12 @@
 // (leading-dimension byte offset = one 64-channel block = 8 KB, stride byte offset = 8 pixel rows = 1 KB),
 // and the instruction descriptor carries a_major = b_major = MN.  No transposed copy is ever made.
 //
-// CTA tile: 128 output channels (two 64-channel boxes of Y) x 128 columns (two (tap, 64-channel) units of
-// X, each its own shifted TMA box with zero fill at the borders) x a slice of the pixel range (split-K).
+// CTA tile: 128 output channels (two 64-channel boxes of Y) x 64 * X_UNITS columns (X_UNITS (tap, 64-channel) units
+// of X, each its own shifted TMA box with zero fill at the borders) x a slice of the pixel range (split-K).
 // Partial tiles go to an fp32 workspace [split][phase][n][t*Cx + c]; ipr_wgrad_reduce_f32 adds the splits
 // in a fixed order (deterministic) and scatters into the parameter's own (reference) layout.
 #include "ipr_common.cuh"
 #include "tc_common.cuh"
-#include <stdlib.h>
 
 namespace {
 
@@ -22,8 +21,6 @@ using namespace tc;
 
 constexpr int KB_PIX = 64;                    // pixels per k-block
 constexpr int UNIT_BYTES = KB_PIX * 128;      // one 64-channel x 64-pixel box
-// Tile configuration (template): X_UNITS (tap, 64-channel) units of X per CTA tile -> N = 64*X_UNITS; STAGES smem stages of
-// (2 + X_UNITS) * 8 KB.
 constexpr int NUM_THREADS = 192;
 constexpr int UMMA_K = 16;
 
@@ -36,7 +33,6 @@ struct WgParams {
     int8_t tap_dw[IPR_TG_MAX_PHASES][IPR_TG_MAX_TAPS];
     float *ws;
     int n_phases;
-    long long *dbg;       // optional per-CTA phase timestamps (profiling builds of the probe only)
 };
 
 struct Maps { CUtensorMap y[4]; CUtensorMap x[4]; };
@@ -52,11 +48,9 @@ wgrad_kernel(const __grid_constant__ Maps maps, const WgParams p)
     const uint32_t bar_empty = bar_full + STAGES * 8;
     const uint32_t bar_tmem = bar_empty + STAGES * 8;
     const uint32_t tmem_slot = bar_tmem + 8;
-    constexpr uint32_t TMEM_COLS = X_UNITS <= 1 ? 64 : (X_UNITS == 2 ? 128 : 256);    // power of two >= 64 * X_UNITS
+    constexpr uint32_t TMEM_COLS = X_UNITS == 2 ? 128 : 256;    // power of two >= 64 * X_UNITS
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const long long t_begin = clock64();
-    const int cta_lin = blockIdx.x + gridDim.x * (blockIdx.y + gridDim.y * blockIdx.z);
     const int n_tiles = (p.n_units + X_UNITS - 1) / X_UNITS;
     const int m_blk = blockIdx.x / n_tiles, n_tile = blockIdx.x - m_blk * n_tiles;
     const int split = blockIdx.y, phase = blockIdx.z;
@@ -124,16 +118,13 @@ wgrad_kernel(const __grid_constant__ Maps maps, const WgParams p)
                 umma_commit(bar_empty + 8 * s);
             }
             umma_commit(bar_tmem);
-            if (p.dbg) p.dbg[cta_lin * 8 + 1] = clock64() - t_begin;     // MMA issue loop finished
         }
         __syncwarp();
     } else {
         const int q = warp & 3;
         const int n = m_blk * 128 + q * 32 + lane;        // output channel (row of dW)
         float *dst_row = p.ws + (((size_t)split * p.n_phases + phase) * p.n_pad + n) * p.k_total;
-        if (p.dbg && warp == 2 && lane == 0) p.dbg[cta_lin * 8 + 0] = clock64() - t_begin;   // setup done
         if (num_kb > 0) { mbar_wait_backoff(bar_tmem, 0); tc_fence_after(); }
-        if (p.dbg && warp == 2 && lane == 0) p.dbg[cta_lin * 8 + 2] = clock64() - t_begin;   // accumulator ready
 #pragma unroll 1
         for (int c0 = 0; c0 < 64 * X_UNITS; c0 += 32) {
             const int unit = unit0 + (c0 >> 6);
@@ -154,7 +145,6 @@ wgrad_kernel(const __grid_constant__ Maps maps, const WgParams p)
                                      __uint_as_float(raw[4 * g + 2]), __uint_as_float(raw[4 * g + 3]));
         }
     }
-    if (p.dbg && warp == 2 && lane == 0) { p.dbg[cta_lin * 8 + 3] = clock64() - t_begin; p.dbg[cta_lin * 8 + 4] = num_kb; }
     tc_fence_before();
     __syncthreads();
     if (warp == 1) tmem_dealloc(tmem_base, TMEM_COLS);
@@ -249,25 +239,12 @@ wgrad_reduce_taps_kernel(const float *__restrict__ ws, int splits, int phases, i
     }
 }
 
-// tile configuration: IPR_WGRAD_CFG = 0: N=128, 3 stages (2 CTAs/SM) | 1: N=128, 6 stages | 2: N=256, 4 stages | 3: N=64, 8 stages.
-// Measured on B200 (scripts/wg_sweep.sh): the MN-major tcgen05.mma stream, not the operand loads, paces this kernel
-// (skipping the TMA loads entirely only drops c3 from 45 to 37 us), and two co-resident CTAs interleave their MMA
-// streams better than one deep pipeline, so config 0 with ~2 CTAs per SM is the default.
-int wgrad_config() {
-    static int cfg = -1;
-    if (cfg < 0) {
-        const char *e = getenv("IPR_WGRAD_CFG");
-        cfg = e ? atoi(e) : 0;
-        if (cfg < 0 || cfg > 3) cfg = 0;
-    }
-    return cfg;
-}
-// X units per CTA tile: the widest of {4, 3, 2} that divides the layer's unit count (9-tap layers -> 3, 16-tap / 4-tap
-// layers -> 4): the kernel is paced by TMA requests per MAC, which fall by 25 % going from N = 128 to N = 192 / 256
-// (measured: 1027 -> 1248 cycles per k-block for twice the MACs), provided no tile is left partly empty.
+// Tile configuration: X_UNITS (tap, 64-channel) units of X per CTA tile, i.e. N = 64 * X_UNITS, and as many smem stages
+// of (2 + X_UNITS) * 8 KB as fit in about 200 KB: <2, 6>, <3, 5> or <4, 4>, one CTA per SM.  X_UNITS is the widest of
+// {4, 3, 2} that divides the layer's unit count (9-tap layers -> 3, 16-tap / 4-tap layers -> 4): the kernel is paced by
+// TMA requests per MAC, which fall by 25 % going from N = 128 to N = 192 / 256 (measured: 1027 -> 1248 cycles per
+// k-block for twice the MACs), provided no tile is left partly empty.
 int wgrad_x_units(int n_units) {
-    static const char *e = getenv("IPR_WGRAD_CFG");
-    if (e) { const int c = atoi(e); return c == 2 ? 4 : (c == 3 ? 1 : (c == 4 ? 3 : 2)); }
     if (n_units % 4 == 0) return 4;
     if (n_units % 3 == 0) return 3;
     return 2;
@@ -368,7 +345,6 @@ extern "C" int ipr_wgrad_bf16(const ipr_wgrad_t *d, ipr_stream_t stream)
     p.n_units = d->n_taps * p.x_chunks; p.n_phases = d->n_phases;
     p.kb_per_split = (p.total_kb + d->splits - 1) / d->splits;
     p.ws = d->workspace;
-    { static const char *e = getenv("IPR_WGRAD_DBG_PTR"); p.dbg = e ? (long long *)strtoull(e, nullptr, 0) : nullptr; }
     for (int ph = 0; ph < IPR_TG_MAX_PHASES; ph++) {
         p.y_map[ph] = d->y_map[ph];
         for (int t = 0; t < IPR_TG_MAX_TAPS; t++) {
@@ -390,7 +366,6 @@ extern "C" int ipr_wgrad_bf16(const ipr_wgrad_t *d, ipr_stream_t stream)
     switch (xu) {
         case 4:  return launch_wgrad<4, 4>(maps, p, grid, ipr_cu(stream));
         case 3:  return launch_wgrad<3, 5>(maps, p, grid, ipr_cu(stream));
-        case 1:  return launch_wgrad<1, 8>(maps, p, grid, ipr_cu(stream));
         default: return launch_wgrad<2, 6>(maps, p, grid, ipr_cu(stream));
     }
 }

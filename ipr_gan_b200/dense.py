@@ -10,10 +10,7 @@ import ctypes
 
 import torch
 
-from ._lib import check, lib
-
-MAX_TAPS, MAX_PHASES = 16, 4
-_SM_COUNT_TILES = 120          # want at least this many CTA tiles before widening the N tile
+from ._lib import MAX_PHASES, MAX_TAPS, TapGemm, WGrad, check, lib  # noqa: F401 (MAX_* and the structs re-exported)
 
 # When set to a list, every GEMM launch appends (kind, algorithmic_flops, start_event, end_event): bench.py uses
 # it for the live tensor-roofline measurement (CUDA events on the launching stream).
@@ -43,38 +40,6 @@ def _prof_end(kind, flops, start, l2_bytes=0.0):
 # that bounds the low-arithmetic-intensity tiles (every tile re-reads its A box per tap and its B block per k-block).
 PROFILE_L2 = None
 EPI_LINEAR, EPI_BIAS_LRELU, EPI_MASK, EPI_TANH_NCHW, EPI_LINEAR_F32, EPI_LINEAR_NCHW = 0, 1, 2, 3, 4, 5
-
-
-class TapGemm(ctypes.Structure):
-    """ipr_tapgemm_t"""
-    _fields_ = [
-        ("a", ctypes.c_void_p), ("a_n", ctypes.c_int32), ("a_h", ctypes.c_int32), ("a_w", ctypes.c_int32),
-        ("a_c", ctypes.c_int32), ("a_parity", ctypes.c_int32), ("q_h", ctypes.c_int32), ("q_w", ctypes.c_int32),
-        ("b", ctypes.c_void_p), ("n_total", ctypes.c_int32), ("block_n", ctypes.c_int32),
-        ("n_phases", ctypes.c_int32), ("n_taps", ctypes.c_int32),
-        ("tap_map", (ctypes.c_int8 * MAX_TAPS) * MAX_PHASES), ("tap_dh", (ctypes.c_int8 * MAX_TAPS) * MAX_PHASES),
-        ("tap_dw", (ctypes.c_int8 * MAX_TAPS) * MAX_PHASES),
-        ("epi_mode", ctypes.c_int32), ("slope", ctypes.c_float), ("sigma", ctypes.c_void_p),
-        ("bias", ctypes.c_void_p), ("mask", ctypes.c_void_p), ("out", ctypes.c_void_p),
-        ("out_h", ctypes.c_int32), ("out_w", ctypes.c_int32), ("out_c", ctypes.c_int32),
-        ("out_sh", ctypes.c_int32), ("out_sw", ctypes.c_int32),
-        ("out_oh", ctypes.c_int8 * MAX_PHASES), ("out_ow", ctypes.c_int8 * MAX_PHASES),
-        ("n_valid", ctypes.c_int32), ("stats", ctypes.c_void_p), ("scale", ctypes.c_void_p),
-    ]
-
-
-
-def _bind():
-    L = lib()
-    if not getattr(L, "_tg_bound", False):
-        L.ipr_tapgemm_bf16.restype = ctypes.c_int
-        L.ipr_tapgemm_bf16.argtypes = [ctypes.POINTER(TapGemm), ctypes.c_void_p]
-        L.ipr_tapgemm_m_tiles.restype = ctypes.c_int
-        L.ipr_tapgemm_m_tiles.argtypes = [ctypes.POINTER(TapGemm)]
-        L.ipr_tapgemm_stats_rows.restype = ctypes.c_int
-        L.ipr_tapgemm_stats_rows.argtypes = [ctypes.POINTER(TapGemm)]
-        L._tg_bound = True
-    return L
 
 
 # stride-2, k=4, pad=1: kernel row kh reads input row 2*o + kh - 1 = 2*(o + d) + parity
@@ -161,7 +126,7 @@ class Plan(object):
     def run(self, a, b_packed, epi=EPI_LINEAR, slope=0.0, sigma=None, bias=None, mask=None, out=None,
             want_stats=False, n_valid=None, out_nchw_c=None, scale=None):
         """a: (N, H, W, C) bf16 NHWC.  Returns (out, stats or None)."""
-        L = _bind()
+        L = lib()
         assert a.dtype == torch.bfloat16 and a.is_cuda and a.is_contiguous() and a.dim() == 4
         N, H, W, C = a.shape
         assert C == self.cin, (C, self.cin)
@@ -249,20 +214,6 @@ class Plan(object):
         return getattr(self, "k_valid_override", self.cin)
 
 
-class WGrad(ctypes.Structure):
-    """ipr_wgrad_t"""
-    _fields_ = [
-        ("y", ctypes.c_void_p), ("y_c", ctypes.c_int32), ("y_parity", ctypes.c_int32),
-        ("x", ctypes.c_void_p), ("x_c", ctypes.c_int32), ("x_parity", ctypes.c_int32),
-        ("n_imgs", ctypes.c_int32), ("q_h", ctypes.c_int32), ("q_w", ctypes.c_int32),
-        ("n_phases", ctypes.c_int32), ("n_taps", ctypes.c_int32),
-        ("y_map", ctypes.c_int8 * MAX_PHASES),
-        ("tap_map", (ctypes.c_int8 * MAX_TAPS) * MAX_PHASES), ("tap_dh", (ctypes.c_int8 * MAX_TAPS) * MAX_PHASES),
-        ("tap_dw", (ctypes.c_int8 * MAX_TAPS) * MAX_PHASES),
-        ("workspace", ctypes.c_void_p), ("splits", ctypes.c_int32),
-    ]
-
-
 _SM_COUNT_CACHE = []
 
 
@@ -275,7 +226,11 @@ def _sm_count():
             n = torch.cuda.get_device_properties(torch.cuda.current_device()).multi_processor_count
         _SM_COUNT_CACHE.append(n)
     return _SM_COUNT_CACHE[0]
-_WGRAD_OVERSUB = int(__import__('os').environ.get('IPR_WGRAD_OVERSUB', '1'))
+
+
+# Weight matrices with at least this many (row, input channel) pairs reduce their split-K partials destination-major
+# (ipr_wgrad_reduce_taps_f32); smaller ones, with many splits and few threads, are faster element-major.
+_REDUCE_TAPS_MIN = 32768
 
 
 class WGradPlan(object):
@@ -323,11 +278,8 @@ class WGradPlan(object):
             for ph, taps in enumerate(fwd.taps):
                 for t, (_, _, _, kh, kw) in enumerate(taps):
                     tap_of[kh * ksz + kw] = ph * self.n_taps + t
-            # only where it pays: big weight matrices (enough (n, c) threads) -- small ones with many splits are
-            # faster element-major
             if kk == self.n_phases * self.n_taps and min(tap_of) >= 0 and row_perm is None and \
-                    self.rows * self.x_c >= int(__import__("os").environ.get("IPR_WGRAD_TAPS_MIN", "32768")) and \
-                    __import__('os').environ.get('IPR_WGRAD_REDUCE_TAPS', '1') != '0':
+                    self.rows * self.x_c >= _REDUCE_TAPS_MIN:
                 self.tap_of = (ctypes.c_int32 * kk)(*tap_of)
                 self.kk = kk
                 if k == "convT4s2":
@@ -343,13 +295,7 @@ class WGradPlan(object):
         return self._dev[key]
 
     def run(self, y, x, grad, accumulate=False, scale=1.0, splits=None):
-        L = _bind()
-        if not getattr(L, "_wg_bound", False):
-            L.ipr_wgrad_bf16.argtypes = [ctypes.POINTER(WGrad), ctypes.c_void_p]
-            L.ipr_wgrad_workspace_bytes.argtypes = [ctypes.POINTER(WGrad)]
-            L.ipr_wgrad_total_kblocks.argtypes = [ctypes.POINTER(WGrad)]
-            L.ipr_wgrad_tiles.argtypes = [ctypes.POINTER(WGrad)]
-            L._wg_bound = True
+        L = lib()
         assert y.dtype == torch.bfloat16 and x.dtype == torch.bfloat16 and y.is_contiguous() and x.is_contiguous()
         assert grad.dtype == torch.float32 and grad.is_contiguous()
         N, xh, xw, xc = x.shape
@@ -373,10 +319,9 @@ class WGradPlan(object):
         if kblocks < 0:
             check(kblocks, "ipr_wgrad_total_kblocks")
         if splits is None:
-            tiles = L.ipr_wgrad_tiles(ctypes.byref(d))           # one CTA per SM (48 KB stages): fill the chip once
-            # one CTA per SM (about 190 KB of smem stages): never exceed one wave, a second partial wave doubles the time
-            slots = _sm_count() * _WGRAD_OVERSUB
-            splits = max(1, min(kblocks // 4 if kblocks >= 8 else 1, slots // tiles, _sm_count()))
+            tiles = L.ipr_wgrad_tiles(ctypes.byref(d))
+            # one CTA per SM (about 200 KB of smem stages): never exceed one wave, a second partial wave doubles the time
+            splits = max(1, min(kblocks // 4 if kblocks >= 8 else 1, _sm_count() // tiles))
         d.splits = splits
         nbytes = L.ipr_wgrad_workspace_bytes(ctypes.byref(d))
         ws = torch.empty(nbytes // 4, device=x.device, dtype=torch.float32)

@@ -62,6 +62,40 @@ def test_convT4s2_forward_with_stats(B, C, O, H):
     close(s[1], (want * want).sum((0, 2, 3)), tol=2e-3)
 
 
+@pytest.mark.parametrize("epi", ["linear", "mask"])
+def test_short_main_loop_stats(epi):
+    """Statistics of a one-k-block layer with one N block and at least 4 tiles per SM: the launch runs a variant whose
+    per-CTA statistics rows must match what ipr_tapgemm_stats_rows allocated.  The stats tensor is handed the block of
+    a freed NaN-filled tensor, so a row the kernel does not write turns the sums into NaN."""
+    from ipr_gan_b200 import dense
+    torch.manual_seed(5)
+    B, C, O, H = 512, 64, 128, 16
+    x = torch.randn(B, H, H, C, device="cuda")
+    w = torch.randn(O, C, device="cuda") * 0.05
+    plan = dense.Plan("linear", C, O)
+    wp = plan.pack(w)
+    kw = dict(want_stats=True)
+    if epi == "mask":
+        mask = torch.randn(B, H, H, O, device="cuda").to(torch.bfloat16)
+        kw.update(epi=dense.EPI_MASK, slope=0.1, mask=mask)
+    a = x.to(torch.bfloat16)
+    out, stats = plan.run(a, wp, **kw)
+    shape = stats.shape
+    del out, stats
+    torch.cuda.synchronize()
+    torch.cuda.empty_cache()
+    torch.full(shape, float("nan"), device="cuda")          # freed at once: its block goes back to the cache
+    out, stats = plan.run(a, wp, **kw)
+    want = (bf(x) @ bf(w).t()).view(B, H, H, O)
+    if epi == "mask":
+        want = want * torch.where(mask.float() > 0, 1.0, 0.1)
+    close(out.float(), want)
+    s = stats.sum(0)
+    close(s[0], want.sum((0, 1, 2)), tol=2e-3)
+    if epi == "linear":
+        close(s[1], (want * want).sum((0, 1, 2)), tol=2e-3)
+
+
 def test_convT3_tanh_nchw():
     from ipr_gan_b200 import dense
     torch.manual_seed(1)
