@@ -179,8 +179,9 @@ class CycleGAN(Model):
         self.real_A, self.real_B = data["real_A"], data["real_B"]
         if data.get("pooled", False):      # the caller already exchanged the images with the history pools
             self.fake_A, self.fake_B = data["fake_A"], data["fake_B"]      # (trainer.ProtectedCycleGANTrainer)
-        else:
-            self.fake_A, self.fake_B = self.poolA(data["fake_A"]), self.poolB(data["fake_B"])
+        else:                              # several ranks: the pools see the gathered global batch
+            from ipr_gan_b200 import dist
+            self.fake_A, self.fake_B = dist.pool_query(self.poolA, data["fake_A"]), dist.pool_query(self.poolB, data["fake_B"])
         st = self._pair_streams()
         if st is None:
             self.RA_logits, self.FA_logits = self.DB(self.real_A), self.DB(self.fake_A.detach())

@@ -29,7 +29,7 @@ def _nvtx(name):
 
 import models  # noqa: E402
 from configs import presets  # noqa: E402
-from ipr_gan_b200 import _lib, engine  # noqa: E402
+from ipr_gan_b200 import _lib, dist, engine  # noqa: E402
 
 
 class ProtectedDCGANTrainer(object):
@@ -155,6 +155,14 @@ class ProtectedDCGANTrainer(object):
 
 
 # ------------------------------------------------------------------------------------------ SRGAN / CycleGAN
+# Data parallelism as for the DCGAN: one process per GPU, each trainer built with its PER-RANK batch and fed its
+# ``dist.shard`` of the global batch; FlatAdam all-reduces the gradient arenas inside the captured graphs.
+def _check_shard(host, static):
+    """A shard of another size would be broadcast or refused by copy_ further down: say what is wrong instead."""
+    if tuple(host.shape) != tuple(static.shape):
+        raise ValueError("expected this rank's shard of shape %s, got %s" % (tuple(static.shape), tuple(host.shape)))
+
+
 def _capture(fn, device, warmup=3, stream=None):
     """Warm ``fn`` up eagerly on a side stream, then capture it into a CUDA graph (weight packing included).
     Warm-up and capture use the SAME stream: autograd's AccumulateGrad nodes remember the stream they were created
@@ -218,11 +226,14 @@ class ProtectedSRGANTrainer(object):
                 self._step()
 
     def step_from_host(self, low_res_cpu, high_res_cpu):
-        """Host batch in, metrics dict out (one step of experiments/image_super_resolution.py's training loop)."""
+        """This rank's host batch in, metrics dict out (one step of experiments/image_super_resolution.py's training
+        loop).  With several ranks the metrics are the global-batch values, the same dict on every rank."""
+        _check_shard(low_res_cpu, self.low_res)
+        _check_shard(high_res_cpu, self.high_res)
         self.low_res.copy_(low_res_cpu, non_blocking=True)
         self.high_res.copy_(high_res_cpu, non_blocking=True)
         self.step()
-        return self.model.get_metrics()
+        return dist.reduce_metrics(self.model.get_metrics())
 
 
 class ProtectedCycleGANTrainer(object):
@@ -232,17 +243,23 @@ class ProtectedCycleGANTrainer(object):
     pool exchange running eagerly between them on static buffers.  The learning rate is a launch argument of the Adam
     kernel: when the schedulers change it (once per epoch) the graphs are re-captured."""
 
-    def __init__(self, device, size=128, seed=1234, use_graph=True):
-        self.device, self.size, self.use_graph = device, size, use_graph
+    def __init__(self, device, size=128, seed=1234, use_graph=True, batch=1):
+        self.device, self.size, self.use_graph, self.batch = device, size, use_graph, batch
+        # the seed also keeps the host RNG of all ranks in lockstep: the image pools draw from it (dist.pool_query)
         torch.manual_seed(seed)
         model = models.CycleGAN(presets.cyclegan_model(), device=[device])
         model = models.BlackBoxWrapper(model, presets.cyclegan_blackbox())
         self.model = models.WhiteBoxWrapper(model, presets.whitebox("GB"))
         self.inner = model.model
-        self.real_A = torch.zeros(1, 3, size, size, device=device)
-        self.real_B = torch.zeros(1, 3, size, size, device=device)
-        self.pooled_A = torch.zeros(1, 3, size, size, device=device)
-        self.pooled_B = torch.zeros(1, 3, size, size, device=device)
+        shape = (batch, 3, size, size)
+        self.real_A = torch.zeros(shape, device=device)
+        self.real_B = torch.zeros(shape, device=device)
+        self.pooled_A = torch.zeros(shape, device=device)
+        self.pooled_B = torch.zeros(shape, device=device)
+        # several ranks: the pools are queried with the global batch, gathered into these
+        w = dist.world()
+        self.gathered_A = torch.zeros((w * batch,) + shape[1:], device=device) if w > 1 else None
+        self.gathered_B = torch.zeros((w * batch,) + shape[1:], device=device) if w > 1 else None
         self.graph_g = self.graph_d = None
         self.launches_per_step = None
         self._lr = None
@@ -260,8 +277,8 @@ class ProtectedCycleGANTrainer(object):
         # graph mode: the tensors the captured generator update writes (forward_d re-binds m.fake_A / m.fake_B to the
         # pooled images, and no Python runs during a replay to bind them back)
         fake_a, fake_b = self._generated if self._generated is not None else (m.fake_A, m.fake_B)
-        self.pooled_A.copy_(m.poolA(fake_a))
-        self.pooled_B.copy_(m.poolB(fake_b))
+        self.pooled_A.copy_(dist.pool_query(m.poolA, fake_a, self.gathered_A))
+        self.pooled_B.copy_(dist.pool_query(m.poolB, fake_b, self.gathered_B))
 
     def _step_d(self):
         self.model.update_d({"real_A": self.real_A, "real_B": self.real_B, "fake_A": self.pooled_A,
@@ -294,7 +311,9 @@ class ProtectedCycleGANTrainer(object):
     def step(self):
         if self.graph_g is None:
             return self._eager()
-        if self._lrs() != self._lr:                  # the schedulers moved the learning rate: capture it anew
+        # the schedulers moved the learning rate: capture it anew (the rate is the same on every rank, so all ranks
+        # re-capture -- their collectives included -- in the same step)
+        if self._lrs() != self._lr:
             self.capture(warmup=0)
         with _nvtx("ipr.cyclegan.step"):
             self.graph_g.replay()
@@ -302,7 +321,10 @@ class ProtectedCycleGANTrainer(object):
             self.graph_d.replay()
 
     def step_from_host(self, real_a_cpu, real_b_cpu):
+        """This rank's host batch in, metrics dict out; with several ranks the global-batch values on every rank."""
+        _check_shard(real_a_cpu, self.real_A)
+        _check_shard(real_b_cpu, self.real_B)
         self.real_A.copy_(real_a_cpu, non_blocking=True)
         self.real_B.copy_(real_b_cpu, non_blocking=True)
         self.step()
-        return self.model.get_metrics()
+        return dist.reduce_metrics(self.model.get_metrics())
