@@ -31,6 +31,18 @@ import models  # noqa: E402
 from configs import presets  # noqa: E402
 from ipr_gan_b200 import _lib, dist, engine  # noqa: E402
 
+# the wrappers' own switches for a step without the trigger pass, the watermark loss and the sign loss
+# (models/protect.py): the plain GAN step of the inner model, which is what the fine-tuning attack trains
+INHIBIT = {"inhibit_bbox": True, "inhibit_wbox": True}
+
+
+def _replayed(*optimizers):
+    """A replay ran these optimizers' Adam launches with no Python around them: bump their arenas' versions, so that
+    the next eager forward re-packs its bf16 GEMM operands (``engine.PackSet``) from the updated masters instead of
+    using the pack the replay wrote before its last optimizer step."""
+    for opt in optimizers:
+        opt.arena.version += 1
+
 
 class ProtectedDCGANTrainer(object):
     def __init__(self, batch, device, seed=1234, fn_inp="TransformDist", use_graph=True, size=32,
@@ -58,6 +70,12 @@ class ProtectedDCGANTrainer(object):
         self.latent_host = torch.zeros(batch, 128).pin_memory()
         self.graph = None
         self.launches_per_step = None
+        # attack switches (robustness.finetune_attack / overwrite_attack): ``inhibit`` runs the inhibited step, and
+        # ``model`` may be replaced by another wrapper stack over the same inner model.  A captured step whose wrapper
+        # stack, inhibit flag or learning rates no longer match is captured anew (the rate is a launch argument).
+        self.inhibit = False
+        self._graph_key = None
+        self.stream = torch.cuda.Stream(device=device)
         # latents drawn on the device (Philox, position kept in device memory): no host randn + H2D copy per step
         # (experiments/image_generation.py:93-96); one stream per rank
         from ipr_gan_b200 import dist, ops
@@ -68,7 +86,11 @@ class ProtectedDCGANTrainer(object):
         if self.normal is not None:
             self.normal.fill_(self.latent)
         self.model.update_d({"real_sample": self.real, "latent": self.latent})
-        self.model.update_g({"fake_sample": self.model.fake_sample})
+        self.model.update_g(dict({"fake_sample": self.model.fake_sample}, **(INHIBIT if self.inhibit else {})))
+
+    def _key(self):
+        m = self.model
+        return id(m), self.inhibit, m.optG.param_groups[0]["lr"], m.optD.param_groups[0]["lr"]
 
     def _step_from_pinned(self):
         """The step preceded by its own input copies (captured as the ``graph_pinned`` variant)."""
@@ -93,8 +115,9 @@ class ProtectedDCGANTrainer(object):
             self.latent.copy_(latent, non_blocking=True)
 
     def capture(self, warmup=3):
-        """Warm up eagerly on a side stream, then capture the step into a CUDA graph."""
-        s = torch.cuda.Stream(device=self.device)
+        """Warm up eagerly on a side stream, then capture the step into a CUDA graph.  The stream is the trainer's
+        own, so that a later re-capture uses the stream autograd's accumulation nodes were created on."""
+        s = self.stream
         s.wait_stream(torch.cuda.current_stream(self.device))
         with torch.cuda.stream(s):
             for _ in range(warmup):
@@ -106,6 +129,7 @@ class ProtectedDCGANTrainer(object):
         if not self.use_graph:
             return
         engine.reset_caches()                       # weight packing must be part of the captured step
+        self._graph_key = self._key()
         self.graph = torch.cuda.CUDAGraph()
         # thread_local: NCCL's watchdog thread may query events while this thread captures (multi-GPU runs)
         with torch.cuda.graph(self.graph, stream=s, capture_error_mode="thread_local"):
@@ -127,7 +151,10 @@ class ProtectedDCGANTrainer(object):
 
     def _step_or_replay(self):
         if self.graph is not None:
+            if self._key() != self._graph_key:
+                self.capture(warmup=0)
             self.graph.replay()
+            _replayed(self.model.optG, self.model.optD)
             board = self.model.board
             if board is not None:
                 board.touch()                       # the replay rewrote the loss slots behind the host's back
@@ -137,6 +164,8 @@ class ProtectedDCGANTrainer(object):
     def step_from_host(self, real_cpu, latent_cpu=None):
         """The call a user of the reference makes (experiments/image_generation.py:92-101): host tensors in,
         metrics dict (Python floats) out.  With ``device_latents`` the latent argument is not needed."""
+        if self.graph_pinned is not None and self._key() != self._graph_key:
+            self.capture(warmup=0)
         if self.graph_pinned is not None:
             # batches normally arrive IN the pinned buffers (no host copy); anything else is staged through them.  The
             # previous step's copies have completed: every call ends with the metrics read-back.
@@ -146,6 +175,7 @@ class ProtectedDCGANTrainer(object):
                 self.latent_host.copy_(latent_cpu)
             with _nvtx("ipr.dcgan.step"):
                 self.graph_pinned.replay()
+                _replayed(self.model.optG, self.model.optD)
                 if self.model.board is not None:
                     self.model.board.touch()
             return self.model.get_metrics()
@@ -202,16 +232,26 @@ class ProtectedSRGANTrainer(object):
         self.low_res = torch.zeros(batch, 3, 24, 24, device=device)
         self.high_res = torch.zeros(batch, 3, 96, 96, device=device)
         self.graph, self.launches_per_step = None, None
+        # attack switches, as on ProtectedDCGANTrainer
+        self.inhibit = False
+        self._graph_key = None
+        self.stream = torch.cuda.Stream(device=device)
 
     def _step(self):
         m = self.model
-        m.update_g({"low_res": self.low_res, "high_res": self.high_res, "pretrain": self.pretrain})
+        m.update_g(dict({"low_res": self.low_res, "high_res": self.high_res, "pretrain": self.pretrain},
+                        **(INHIBIT if self.inhibit else {})))
         if not self.pretrain:
             m.update_d({"high_res": m.high_res, "super_res": m.super_res})
 
+    def _key(self):
+        m = self.model
+        return id(m), self.inhibit, m.optG.param_groups[0]["lr"], m.optD.param_groups[0]["lr"]
+
     def capture(self, warmup=3):
         if self.use_graph:
-            self.graph, self.launches_per_step = _capture(self._step, self.device, warmup)
+            self._graph_key = self._key()
+            self.graph, self.launches_per_step = _capture(self._step, self.device, warmup, stream=self.stream)
         else:
             for _ in range(warmup):
                 before = _lib.launch_count()
@@ -221,7 +261,10 @@ class ProtectedSRGANTrainer(object):
     def step(self):
         with _nvtx("ipr.srgan.step"):
             if self.graph is not None:
+                if self._key() != self._graph_key:
+                    self.capture(warmup=0)
                 self.graph.replay()
+                _replayed(self.model.optG, self.model.optD)
             else:
                 self._step()
 
@@ -262,15 +305,18 @@ class ProtectedCycleGANTrainer(object):
         self.gathered_B = torch.zeros((w * batch,) + shape[1:], device=device) if w > 1 else None
         self.graph_g = self.graph_d = None
         self.launches_per_step = None
-        self._lr = None
+        self._graph_key = None
         self._generated = None
         self.stream = torch.cuda.Stream(device=device)
+        # attack switches, as on ProtectedDCGANTrainer (``inner`` stays the model every wrapper stack wraps)
+        self.inhibit = False
 
-    def _lrs(self):
-        return (self.inner.optG.param_groups[0]["lr"], self.inner.optD.param_groups[0]["lr"])
+    def _key(self):
+        return (id(self.model), self.inhibit, self.inner.optG.param_groups[0]["lr"],
+                self.inner.optD.param_groups[0]["lr"])
 
     def _step_g(self):
-        self.model.update_g({"real_A": self.real_A, "real_B": self.real_B})
+        self.model.update_g(dict({"real_A": self.real_A, "real_B": self.real_B}, **(INHIBIT if self.inhibit else {})))
 
     def _pool(self):
         m = self.inner
@@ -306,19 +352,21 @@ class ProtectedCycleGANTrainer(object):
             self._generated = (self.inner.fake_A, self.inner.fake_B)
             self.graph_d, n_d = _capture(self._step_d, self.device, 0, stream=s)
             self.launches_per_step = n_g + n_d
-            self._lr = self._lrs()
+            self._graph_key = self._key()
 
     def step(self):
         if self.graph_g is None:
             return self._eager()
-        # the schedulers moved the learning rate: capture it anew (the rate is the same on every rank, so all ranks
-        # re-capture -- their collectives included -- in the same step)
-        if self._lrs() != self._lr:
+        # the schedulers moved the learning rate, or an attack switched the step: capture it anew (the rate is the
+        # same on every rank, so all ranks re-capture -- their collectives included -- in the same step)
+        if self._key() != self._graph_key:
             self.capture(warmup=0)
         with _nvtx("ipr.cyclegan.step"):
             self.graph_g.replay()
+            _replayed(self.inner.optG)
             self._pool()
             self.graph_d.replay()
+            _replayed(self.inner.optD)
 
     def step_from_host(self, real_a_cpu, real_b_cpu):
         """This rank's host batch in, metrics dict out; with several ranks the global-batch values on every rank."""
